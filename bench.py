@@ -2,6 +2,7 @@
 """bench.py — RK4 sample-steps/sec of the closed-loop rollout (BASELINE.json metric) on N B200s of one box.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--workload swarm50|swap12|singlequad|...] [--impl reference]
+                    [--dump-outputs DIR]
 
 A "step" is one OCflow call (mean mode) over one batch of synthetic initial states drawn from the problem's initial
 distribution (SURVEY.md 8d).  The DEFAULT workload is the north_star's target shape, BASELINE.json configs[3]: the swarm50
@@ -480,6 +481,15 @@ def measure(workload, n, steps, warmup, device, dtype, dist, rank, world, seed_r
     return out
 
 
+def dump_outputs(out_dir, sums, Jc, cs):
+    """What the last timed step returned, so that two builds can be compared output for output on the same seeded inputs:
+    sums.npy = the float64 vector [sum L, G, HJt, HJfin, HJgrad, Q, W, row count] of ocflow_sums (after the all-reduce), and
+    costs.npy = [Jc, L, G, HJt, HJfin, HJgrad, Q, W], the objective and mean costs OCflow returns, in the workload's precision."""
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "sums.npy"), sums.cpu().numpy().astype(np.float64))
+    np.save(os.path.join(out_dir, "costs.npy"), torch.stack([Jc] + list(cs)).cpu().numpy())
+
+
 def shard(total, world, rank):
     """rows [lo, hi) of rank `rank`: contiguous blocks of ceil(total / world) rows (neuraloc_b200.sharded.shard_rows)."""
     per = -(-total // world)
@@ -500,7 +510,12 @@ def main():
     ap.add_argument("--latency", action="store_true", help="batch-1 rollout latency (timeDeployment/timeOC.py protocol) instead of throughput")
     ap.add_argument("--train", action="store_true", help="time one training evaluation: OCflow in train mode + Jc.backward() (SURVEY.md 8f N1)")
     ap.add_argument("--intermediates", action="store_true", help="time OCflow(..., intermediates=True): trajectories + controls written to HBM (SURVEY.md 8f N2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed step as DIR/<name>.npy (throughput measurement)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.latency or args.intermediates or args.train):
+        ap.error("--dump-outputs applies to the throughput measurement only")
     W = WORKLOADS[args.workload]
     nt = W["nt"]
     dtype = torch.float32 if W["dtype"] == "f32" else torch.float64
@@ -578,6 +593,8 @@ def main():
         nb._cabi.check(lib.noc_measure_fma_peak(0 if W["dtype"] == "f32" else 1, pk))
         peak = pk.value
         Jc, cs = nb.costs_from_sums(m["sums"], m["alph"], dtype)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, m["sums"], Jc, cs)
         e2e_Jc = float(nb.costs_from_sums(m["e2e_sums"], m["alph"], dtype)[0])
         sub = ""
         if W.get("full_n") and total != W["full_n"]:

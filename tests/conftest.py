@@ -12,7 +12,7 @@ GOLDEN = os.path.join(ROOT, "tests", "golden")
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box via gpurun)")
-    config.addinivalue_line("markers", "reference: needs the read-only reference checkout at /root/reference")
+    config.addinivalue_line("markers", "reference: needs a checkout of the original NeuralOC project, named by NOC_REFERENCE")
 
 
 @pytest.fixture(scope="session")

@@ -372,3 +372,34 @@ def test_batched_shock_restart(nb, monkeypatch):
     with torch.no_grad():
         one = nb.OCflow_shock(x[:3].cuda(), net, prob, nt, [0.1, shock[:1]], "rk4", meta["alph"])  # a [1,d] shock row broadcasts
     assert one[2].shape == (3, 8, 47)
+
+
+def test_bench_dump_outputs_are_the_timed_steps_results(nb, tmp_path):
+    """bench.py --dump-outputs: two runs with different --steps time that many steps (launches scale with it) and dump the same
+    arrays, which are what ocflow_sums returns for the bench's seeded batch and what OCflow derives from them."""
+    import importlib.util
+    runs = {}
+    for steps in (2, 5):
+        out = tmp_path / ("s%d" % steps)
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--workload", "swap12", "--samples", "8192",
+                            "--steps", str(steps), "--warmup", "1", "--no-cpu-baseline", "--dump-outputs", str(out)],
+                           capture_output=True, text=True, cwd=str(tmp_path), timeout=600)
+        assert p.returncode == 0, p.stderr[-2000:]
+        line = json.loads(p.stdout.strip().splitlines()[-1])
+        runs[steps] = (line, np.load(out / "sums.npy"), np.load(out / "costs.npy"))
+    (l2, s2, c2), (l5, s5, c5) = runs[2], runs[5]
+    assert (l2["steps"], l5["steps"]) == (2, 5) and l2["gpu_launches"] > 0 and 2 * l5["gpu_launches"] == 5 * l2["gpu_launches"]
+    assert s2.dtype == np.float64 and s2.shape == (8,) and c2.dtype == np.float32 and c2.shape == (8,)
+    assert np.array_equal(s2, s5) and np.array_equal(c2, c5) and s2[7] == 8192
+    assert float(c2[0]) == l2["config"]["Jc"]
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    device = torch.device("cuda", 0)
+    net, prob, xinit, meta = b.build_case("swap12", device, torch.float32)
+    x = b.sample_x("swap12", xinit, meta["var0"], 8192, 1234, device, torch.float32)
+    with torch.no_grad():
+        sums = nb.ocflow_sums(x, net, prob, [0.0, 1.0], b.WORKLOADS["swap12"]["nt"], "rk4", meta["alph"])
+    Jc, cs = nb.costs_from_sums(sums, meta["alph"], torch.float32)
+    assert np.array_equal(sums.cpu().numpy(), s2)
+    assert np.array_equal(torch.stack([Jc] + cs).cpu().numpy(), c2)

@@ -118,15 +118,25 @@ def test_descriptor_flattening_and_guards():
     assert [float(c) for c in cs] == [5.0, 1.0, 2.0, 3.0, 4.0, 0.5, 1.5] and float(Jc) == 5 + 2 * 1 + 3 * 2 + 4 * 3 + 5 * 4
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not os.path.isdir("/root/reference/src"), reason="reference checkout not present")
-def test_dropin_hook_rebinds_reference_module():
-    """PYTHONPATH=dropin:repo:reference -> `from src.OCflow import OCflow` is the B200 implementation (INTEGRATION.md §1)."""
-    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "neuraloc_b200", "dropin"), ROOT, "/root/reference"]))
+def test_dropin_hook_rebinds_reference_module(tmp_path):
+    """PYTHONPATH=dropin:repo:reference -> `from src.OCflow import OCflow` is the B200 implementation (INTEGRATION.md §1).
+    The reference checkout is not part of this repository: a stand-in `src` package with the reference's module and entry-point
+    names takes its place, so the hook is exercised the way the reference scripts import."""
+    src = tmp_path / "src"
+    src.mkdir()
+    (src / "__init__.py").write_text("")
+    (src / "OCflow.py").write_text(
+        "def OCflow(*a, **k):\n    raise AssertionError('the stand-in reference OCflow ran')\n"
+        "stepRK4 = stepRK1 = ocOdefun = OCflow\n"
+        "def ocG(z, xtarget):\n    return z[:, :xtarget.shape[0]] - xtarget\n")
+    (src / "Phi.py").write_text("class Phi:\n    pass\n")
+    (src / "initProb.py").write_text("def initProb(*a, **k):\n    raise NotImplementedError\n")
+    env = dict(os.environ, PYTHONPATH=os.pathsep.join([os.path.join(ROOT, "neuraloc_b200", "dropin"), ROOT, str(tmp_path)]))
     code = ("from src.OCflow import OCflow, stepRK4, ocG; import src.OCflow as m, neuraloc_b200 as nb;"
             "assert OCflow is nb.OCflow and stepRK4 is nb.stepRK4; assert m._reference_OCflow is not None;"
+            "assert m.stepRK1 is nb.stepRK1 and m.ocOdefun is nb.ocOdefun and m._reference_OCflow.__module__ == 'src.OCflow';"
             "from src.Phi import Phi; from src.initProb import initProb; print('hooked')")
-    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd="/tmp")
+    out = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, cwd=str(tmp_path))
     assert out.returncode == 0 and "hooked" in out.stdout, out.stderr
 
 
@@ -152,6 +162,29 @@ def test_bench_flop_accounting():
     for world in (1, 2, 3, 8):
         rows = [b.shard(1000003, world, r) for r in range(world)]
         assert rows[0][0] == 0 and rows[-1][1] == 1000003 and all(rows[i][1] == rows[i + 1][0] for i in range(world - 1))
+
+
+def test_bench_dump_outputs_format_and_argument_checks(tmp_path):
+    """bench.py --dump-outputs writes the cost sums (float64) and [Jc, cs] in the workload's precision; it refuses the modes it
+    does not cover and a step count below one before touching the GPU."""
+    import importlib.util
+    spec = importlib.util.spec_from_file_location("bench_mod", os.path.join(ROOT, "bench.py"))
+    b = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(b)
+    sums = torch.tensor([10.0, 2.0, 4.0, 6.0, 8.0, 1.0, 3.0, 2.0], dtype=torch.float64)
+    for dtype, npt in ((torch.float32, np.float32), (torch.float64, np.float64)):
+        Jc, cs = nb.costs_from_sums(sums, [2.0, 0, 0, 3.0, 4.0, 5.0], dtype)
+        b.dump_outputs(str(tmp_path / "out"), sums, Jc, cs)
+        s, c = np.load(tmp_path / "out" / "sums.npy"), np.load(tmp_path / "out" / "costs.npy")
+        assert s.dtype == np.float64 and np.array_equal(s, sums.numpy())
+        assert c.dtype == npt and c.tolist() == [45.0, 5.0, 1.0, 2.0, 3.0, 4.0, 0.5, 1.5]
+    for extra in (["--latency"], ["--train"], ["--intermediates"], ["--impl", "reference"]):
+        p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--dump-outputs", str(tmp_path / "x")] + extra,
+                           capture_output=True, text=True, cwd=str(tmp_path))
+        assert p.returncode == 2 and "--dump-outputs" in p.stderr, (extra, p.stderr[-500:])
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "0"], capture_output=True, text=True, cwd=str(tmp_path))
+    assert p.returncode == 2 and "--steps" in p.stderr
+    assert not (tmp_path / "x").exists()
 
 
 def test_bench_does_not_import_test_helpers_or_oracle_at_import():

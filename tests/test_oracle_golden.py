@@ -19,11 +19,47 @@ def _mean_vec(out):
     return np.array([float(Jc)] + [float(c) for c in cs])
 
 
-def _check_costs(got, ref, tol, what):
+def _fp32_noise(c, key, tag, axes=()):
+    """Twice the reference's own fp32 rounding on fixture `key`: 2 |fp32 run - fp64 run| per entry, or its maximum over
+    `axes` (e.g. over the samples and control components of one time step); zeros for fp64.  fp32 sums round differently
+    with the host's BLAS kernels and thread count, so the oracle's fp32 run on another machine differs from the stored
+    fp32 run by rounding of that size."""
+    r32, r64 = np.asarray(c[key + "f32"], dtype=np.float64), np.asarray(c[key + "f64"], dtype=np.float64)
+    d = 2 * np.abs(r32 - r64) if tag == "f32" else np.zeros_like(r64)
+    return d.max(axis=axes, keepdims=True) if axes != () else d
+
+
+def _truth(c, key, tag, sl=np.s_[...]):
+    """The reference's fp64 run of fixture `key` for fp32 checks (see _entry_err); None for fp64."""
+    return c[key + "f64"][sl] if tag == "f32" else None
+
+
+def _check_costs(got, ref, tol, what, noise):
     got, ref = np.asarray(got, dtype=np.float64), np.asarray(ref, dtype=np.float64)
     err = np.abs(got - ref) / np.maximum(np.abs(ref), 1e-30)
-    ok = (err <= tol["cost"]) | (np.abs(got - ref) <= tol["abs"])
+    ok = (err <= tol["cost"]) | (np.abs(got - ref) <= np.maximum(tol["abs"], noise))
     assert ok.all(), "%s: got %s ref %s relerr %s" % (what, got, ref, err)
+
+
+def _state_ok(z, c, key, tag, tol, d):
+    """Within the state tolerance of the stored run in the same precision; in fp32, alternatively within twice the
+    reference's own fp32 distance from its fp64 run, of either of its runs (fp32 rounding follows the host, see _fp32_noise)."""
+    if rel_state_err(z, c[key + tag], d) <= tol["state"]:
+        return True
+    if tag != "f32":
+        return False
+    noise = 2 * rel_state_err(c[key + "f32"], c[key + "f64"], d)
+    return min(rel_state_err(z, c[key + "f32"], d), rel_state_err(z, c[key + "f64"], d)) <= noise
+
+
+def _entry_err(got, ref, rel, floor, noise=0.0, truth=None):
+    """max over entries of |got - ref| / max(rel * max(|ref|, floor), noise): the check passes at <= 1.  With the reference's
+    fp64 run as `truth` (fp32 checks), an entry may instead be within `noise` of that run, as for the states (_state_ok)."""
+    got, ref = np.asarray(got, dtype=np.float64), np.asarray(ref, dtype=np.float64)
+    err = np.abs(got - ref) / np.maximum(rel * np.maximum(np.abs(ref), floor), np.maximum(noise, 1e-300))
+    if truth is not None:
+        err = np.minimum(err, np.abs(got - np.asarray(truth, dtype=np.float64)) / np.maximum(noise, 1e-300))
+    return float(err.max())
 
 
 @pytest.mark.parametrize("tag", ["f32", "f64"])
@@ -36,11 +72,12 @@ def test_rollout_at_xinit(name, tag):
     with torch.no_grad():
         mean = _mean_vec(orc.ocflow(xinit, P, D, [0.0, 1.0], nt, "rk4", meta["alph"]))
         zf, cf = orc.ocflow(xinit, P, D, [0.0, 1.0], nt, "rk4", meta["alph"], intermediates=True)
-    _check_costs(mean, c["xinit_mean_" + tag], tol, "mean costs")
+    _check_costs(mean, c["xinit_mean_" + tag], tol, "mean costs", _fp32_noise(c, "xinit_mean_", tag))
     d = xinit.shape[1]
-    assert rel_state_err(zf.numpy(), c["xinit_z_" + tag], d) <= tol["state"]
+    assert _state_ok(zf.numpy(), c, "xinit_z_", tag, tol, d)
     assert zf.shape == c["xinit_z_" + tag].shape and cf.shape == c["xinit_ctrl_" + tag].shape
-    assert rel_err(cf.numpy()[:, :, 1:], c["xinit_ctrl_" + tag][:, :, 1:], floor=1e-3) <= 50 * tol["state"]
+    assert _entry_err(cf.numpy()[:, :, 1:], c["xinit_ctrl_" + tag][:, :, 1:], 50 * tol["state"], 1e-3,
+                      _fp32_noise(c, "xinit_ctrl_", tag, axes=(0, 1))[:, :, 1:], _truth(c, "xinit_ctrl_", tag, np.s_[:, :, 1:])) <= 1
     assert not cf.numpy()[:, :, 0].any()
 
 
@@ -55,13 +92,14 @@ def test_rollout_batch_three_modes(name, tag):
         mean = _mean_vec(orc.ocflow(x, P, D, [0.0, 1.0], nt, "rk4", meta["alph"]))
         Jn, cn = orc.ocflow(x, P, D, [0.0, 1.0], nt, "rk4", meta["alph"], noMean=True)
         zf, cf = orc.ocflow(x, P, D, [0.0, 1.0], nt, "rk4", meta["alph"], intermediates=True)
-    _check_costs(mean, c["b_mean_" + tag], tol, "batch mean")
+    _check_costs(mean, c["b_mean_" + tag], tol, "batch mean", _fp32_noise(c, "b_mean_", tag))
     nomean = np.concatenate([Jn.numpy()] + [v.numpy() for v in cn], axis=1)
     ref = c["b_nomean_" + tag]
     scale = np.maximum(np.abs(ref).max(axis=0, keepdims=True), 1e-30)
-    assert (np.abs(nomean - ref) / scale).max() <= 10 * tol["cost"]
-    assert rel_state_err(zf.numpy(), c["b_z_" + tag], d) <= tol["state"]
-    assert rel_err(cf.numpy(), c["b_ctrl_" + tag], floor=1e-2) <= 100 * tol["state"]
+    noise = _fp32_noise(c, "b_nomean_", tag, axes=0)
+    assert (np.abs(nomean - ref) / np.maximum(10 * tol["cost"] * scale, np.maximum(noise, 1e-300))).max() <= 1
+    assert _state_ok(zf.numpy(), c, "b_z_", tag, tol, d)
+    assert _entry_err(cf.numpy(), c["b_ctrl_" + tag], 100 * tol["state"], 1e-2, _fp32_noise(c, "b_ctrl_", tag, axes=(0, 1)), _truth(c, "b_ctrl_", tag)) <= 1
 
 
 @pytest.mark.parametrize("tag", ["f32", "f64"])
@@ -76,11 +114,11 @@ def test_rk1_and_unknown_stepper(name, tag):
         zf, _ = orc.ocflow(x[:4], P, D, [0.0, 1.0], 8, "rk1", meta["alph"], intermediates=True)
         mean0 = _mean_vec(orc.ocflow(x[:2], P, D, [0.0, 1.0], 3, "none", meta["alph"]))
         z0, c0 = orc.ocflow(x[:2], P, D, [0.0, 1.0], 3, "none", meta["alph"], intermediates=True)
-    _check_costs(mean, c["rk1_mean_" + tag], tol, "rk1 mean")
-    assert rel_state_err(zf.numpy(), c["rk1_z_" + tag], d) <= tol["state"]
-    _check_costs(mean0, c["nostep_mean_" + tag], tol, "no-stepper mean")
-    assert rel_state_err(z0.numpy(), c["nostep_z_" + tag], d) <= tol["state"]
-    assert rel_err(c0.numpy(), c["nostep_ctrl_" + tag], floor=1e-2) <= 100 * tol["state"]
+    _check_costs(mean, c["rk1_mean_" + tag], tol, "rk1 mean", _fp32_noise(c, "rk1_mean_", tag))
+    assert _state_ok(zf.numpy(), c, "rk1_z_", tag, tol, d)
+    _check_costs(mean0, c["nostep_mean_" + tag], tol, "no-stepper mean", _fp32_noise(c, "nostep_mean_", tag))
+    assert _state_ok(z0.numpy(), c, "nostep_z_", tag, tol, d)
+    assert _entry_err(c0.numpy(), c["nostep_ctrl_" + tag], 100 * tol["state"], 1e-2, _fp32_noise(c, "nostep_ctrl_", tag, axes=(0, 1)), _truth(c, "nostep_ctrl_", tag)) <= 1
 
 
 @pytest.mark.parametrize("tag", ["f32", "f64"])
@@ -95,10 +133,10 @@ def test_shock_restart_tspan(tag):
         xs = torch.from_numpy(c["shock2_x_" + tag]).to(DT[tag])
         m2 = _mean_vec(orc.ocflow(xs, P, D, [0.1, 1.0], 1 + nt - nS, "rk4", meta["alph"]))
         z2, c2 = orc.ocflow(xs, P, D, [0.1, 1.0], 1 + nt - nS, "rk4", meta["alph"], intermediates=True)
-    assert rel_state_err(z1.numpy(), c["shock1_z_" + tag], 4) <= tol["state"]
-    assert rel_state_err(z2.numpy(), c["shock2_z_" + tag], 4) <= tol["state"]
-    _check_costs(m2, c["shock2_mean_" + tag], tol, "shock2 mean")
-    assert rel_err(c2.numpy(), c["shock2_ctrl_" + tag], floor=1e-2) <= 100 * tol["state"]
+    assert _state_ok(z1.numpy(), c, "shock1_z_", tag, tol, 4)
+    assert _state_ok(z2.numpy(), c, "shock2_z_", tag, tol, 4)
+    _check_costs(m2, c["shock2_mean_" + tag], tol, "shock2 mean", _fp32_noise(c, "shock2_mean_", tag))
+    assert _entry_err(c2.numpy(), c["shock2_ctrl_" + tag], 100 * tol["state"], 1e-2, _fp32_noise(c, "shock2_ctrl_", tag, axes=(0, 1)), _truth(c, "shock2_ctrl_", tag)) <= 1
 
 
 @pytest.mark.parametrize("tag", ["f32", "f64"])
@@ -117,11 +155,12 @@ def test_problem_functors(tag):
                              training=(mode == "train"))
             L, H, Q, W = orc.lhqw(D, x, p)
             got = np.stack([np.asarray(v).reshape(-1) for v in (L, H, Q, W)], axis=1)
-            ref = z["%s_%s_LHQW" % (key, mode)]
-            scale = np.maximum(np.abs(ref), 1.0)
-            assert (np.abs(got - ref) / scale).max() <= tol, (name, mode)
-            assert rel_err(orc.grad_p_hamiltonian(D, x, p).numpy(), z["%s_%s_gradpH" % (key, mode)], floor=1.0) <= tol
-            assert rel_err(orc.controls(D, x, p).numpy(), z["%s_%s_ctrls" % (key, mode)], floor=1.0) <= tol
+            ref = lambda k: z["%s_%s_%s" % (key, mode, k)]
+            noise = lambda k: _fp32_noise({t: z["%s_%s_%s_%s" % (name, t, mode, k)] for t in ("f32", "f64")}, "", tag)
+            truth = lambda k: z["%s_f64_%s_%s" % (name, mode, k)] if tag == "f32" else None
+            assert _entry_err(got, ref("LHQW"), tol, 1.0, noise("LHQW"), truth("LHQW")) <= 1, (name, mode)
+            assert _entry_err(orc.grad_p_hamiltonian(D, x, p).numpy(), ref("gradpH"), tol, 1.0, noise("gradpH"), truth("gradpH")) <= 1
+            assert _entry_err(orc.controls(D, x, p).numpy(), ref("ctrls"), tol, 1.0, noise("ctrls"), truth("ctrls")) <= 1
 
 
 @pytest.mark.parametrize("tag", ["f32", "f64"])

@@ -1,6 +1,10 @@
-"""Oracle vs the LIVE reference (only where /root/reference exists, i.e. the build container).
+"""Oracle vs the LIVE reference: runs only where the environment variable NOC_REFERENCE names a checkout of the original
+NeuralOC project (the directory holding its `src/`); skipped otherwise.  No such checkout was available when the suite was
+made self-contained, so the fresh-seed outputs this test compares against could not be stored as golden data.  Its main
+comparison, the reference's outputs on seeded batches in both precisions for all five problems, is kept everywhere by the
+stored tests/golden/cases_*.npz in tests/test_oracle_golden.py.
 
-Complements the committed fixtures: fresh seeds, larger batches, every problem name of initProb."""
+With a checkout it adds: fresh seeds, larger batches, every problem name of initProb."""
 import os
 import sys
 
@@ -11,9 +15,10 @@ import torch
 from oracle import ocflow_oracle as orc
 from helpers import PROBLEMS, load_ckpt
 
-REF = os.environ.get("NOC_REFERENCE", "/root/reference")
+REF = os.environ.get("NOC_REFERENCE", "")
 pytestmark = [pytest.mark.reference,
-              pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "src")), reason="reference checkout not present")]
+              pytest.mark.skipif(not (REF and os.path.isdir(os.path.join(REF, "src"))),
+                                 reason="NOC_REFERENCE does not name a checkout of the original NeuralOC project")]
 
 
 @pytest.fixture(scope="module")
