@@ -143,6 +143,25 @@ int noc_ocflow_host(const noc_phi_t* phi, const noc_prob_t* prob, const void* x_
 int noc_phi_eval(const noc_phi_t* phi, const void* s, int64_t n, int32_t dtype,
                  void* out_phi, void* out_grad, void* stream);
 
+/*
+ * noc_phi_vjp — reverse-mode product of Phi.forward (Phi.py:91-96) and Phi.getGrad (Phi.py:99-138) on a batch: what
+ * `torch.autograd.grad` of a loss built from net(s) and net.getGrad(s) needs.  For rows s_i = [x_i, t_i], a seed a on Phi and a
+ * seed B on grad_s Phi, with  psi_i = a_i Phi(s_i) + B_i . grad_s Phi(s_i):
+ *
+ *   s            dev [n, d+1]
+ *   seed_phi     dev [n] (a) or NULL (zero)
+ *   seed_grad    dev [n, d+1] (B) or NULL (zero)
+ *   grad_params  dev [P] or NULL: SUMS over the rows of d psi_i / d parameter, in noc_ocflow_grad's order and length
+ *                (A, c.weight, c.bias, w.weight, N.layers.0.weight, N.layers.0.bias, N.layers.1.weight, N.layers.1.bias).
+ *                Overwritten, not accumulated; floating-point atomics: reproducible to rounding, not bitwise.
+ *   grad_s       dev [n, d+1] or NULL: d psi_i / d s_i = a_i grad Phi(s_i) + Hess Phi(s_i) B_i (last column: d / dt)
+ *
+ * One launch of the training kernel's second-order sweep per call (+ weight packing and the gradient compaction).  nTh == 2
+ * only (NOC_ERR_UNSUPPORTED otherwise), even widths m, fp32 and fp64.
+ */
+int noc_phi_vjp(const noc_phi_t* phi, const void* s, int64_t n, const void* seed_phi,
+                const void* seed_grad, int32_t dtype, void* grad_params, void* grad_s, void* stream);
+
 /* noc_prob_eval — replaces prob.calcLHQW(x,p), prob.calcGradpH(x,p), prob.calcCtrls(x,p) on a batch.
  *   x, p dev [n, d]; out_lhqw dev [n, 4] = (L, H, Q, W); out_gradpH dev [n, d]; out_ctrls dev [n, nCtrl];
  *   any output may be NULL. */

@@ -20,7 +20,7 @@ MODE_MEAN, MODE_NOMEAN, MODE_INTERMEDIATES = 0, 1, 2
 # every symbol include/noc_b200.h declares (tests check the library exports exactly these)
 SYMBOLS = ["noc_version", "noc_last_error", "noc_device_info", "noc_ctrl_dim", "noc_stage_times", "noc_ocflow",
            "noc_ocflow_host", "noc_phi_eval", "noc_prob_eval", "noc_measure_fma_peak", "noc_tc_probe", "noc_launch_count",
-           "noc_last_path", "noc_sample_rho0", "noc_philox_raw", "noc_ocflow_grad", "noc_baseline_loss"]
+           "noc_last_path", "noc_sample_rho0", "noc_philox_raw", "noc_ocflow_grad", "noc_baseline_loss", "noc_phi_vjp"]
 
 
 class PhiT(C.Structure):
@@ -66,6 +66,7 @@ def lib():
                                   vp, vp, vp, vp]
     L.noc_baseline_loss.argtypes = [C.POINTER(ProbT), vp, vp, i64, i32, i32, dbl, i32, vp, vp, vp]
     L.noc_phi_eval.argtypes = [C.POINTER(PhiT), vp, i64, i32, vp, vp, vp]
+    L.noc_phi_vjp.argtypes = [C.POINTER(PhiT), vp, i64, vp, vp, i32, vp, vp, vp]
     L.noc_prob_eval.argtypes = [C.POINTER(ProbT), vp, vp, i64, i32, i32, vp, vp, vp, vp]
     L.noc_measure_fma_peak.argtypes = [i32, C.POINTER(dbl)]
     L.noc_tc_probe.argtypes = [vp, vp, vp, i32, i32, i32, i32, vp]

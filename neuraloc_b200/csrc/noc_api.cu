@@ -867,6 +867,22 @@ static int phi_eval_impl(const noc_phi_t* ph, const void* s, int64_t n, void* ou
 }
 
 template <typename real>
+static int phi_vjp_impl(const noc_phi_t* ph, const void* s, int64_t n, const void* seed_phi, const void* seed_grad, void* grad_params,
+                        void* grad_s, cudaStream_t st) {
+    PhiPack<real> P;
+    PhiRaw<real> R;
+    int rc = fill_phi<real>(ph, P, R);
+    if (rc) return rc;
+    if (ph->nTh != 2) return fail(NOC_ERR_UNSUPPORTED, "noc_phi_vjp: nTh = %d (the reverse-mode product is written for nTh = 2)", ph->nTh);
+    if (!s || n < 1) return fail(NOC_ERR_ARG, "s is NULL or n < 1");
+    if (!grad_params && !grad_s) return NOC_OK;
+    rc = device_facts();
+    if (rc) return rc;
+    return phi_vjp<real>(ph->d, ph->m, ph->r, (double)P.h, R, (const real*)s, n, (const real*)seed_phi, (const real*)seed_grad,
+                         (real*)grad_params, (real*)grad_s, g_smem_optin, st);
+}
+
+template <typename real>
 static int prob_eval_impl(const noc_prob_t* pb, const void* x, const void* p, int64_t n, int d, void* o_lhqw, void* o_g,
                           void* o_c, cudaStream_t st, int dtype) {
     RolloutArgs<real> A;
@@ -974,6 +990,14 @@ int noc_phi_eval(const noc_phi_t* phi, const void* s, int64_t n, int32_t dtype, 
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == NOC_F32) return phi_eval_impl<float>(phi, s, n, out_phi, out_grad, st, dtype);
     if (dtype == NOC_F64) return phi_eval_impl<double>(phi, s, n, out_phi, out_grad, st, dtype);
+    return fail(NOC_ERR_ARG, "dtype must be NOC_F32 or NOC_F64");
+}
+
+int noc_phi_vjp(const noc_phi_t* phi, const void* s, int64_t n, const void* seed_phi, const void* seed_grad, int32_t dtype,
+                void* grad_params, void* grad_s, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    if (dtype == NOC_F32) return phi_vjp_impl<float>(phi, s, n, seed_phi, seed_grad, grad_params, grad_s, st);
+    if (dtype == NOC_F64) return phi_vjp_impl<double>(phi, s, n, seed_phi, seed_grad, grad_params, grad_s, st);
     return fail(NOC_ERR_ARG, "dtype must be NOC_F32 or NOC_F64");
 }
 

@@ -24,6 +24,8 @@
 //
 // (the beta terms belong to the terminal block, where Phi itself enters |Phi - alpha_0 G|).  Parameter gradients of a tile are
 // reduced over its TS samples in registers and added to the global gradient with one red.global.add per element and evaluation.
+// The same kernel, instantiated with VJP = true, differentiates Phi.forward / Phi.getGrad alone (noc_phi_vjp): the terminal
+// block's two sweeps once per row, gbar and beta read from memory.
 // The L / HJt accumulators of z have constant adjoints (1 and alpha_3), Q and W are reported only (adjoint 0), so the only state
 // adjoint is lambda = dJ/dx, a [d][TS] panel.
 #include "noc_launch.cuh"
@@ -67,6 +69,10 @@ struct GradArgs {
     // shared-memory offsets (elements)
     int o_s, o_g, o_gb, o_q, o_sb, o_xd, o_lam, o_xbn, o_xsum, o_z0, o_za, o_sc, o_red, o_qx, o_as, o_ag, o_bt, o_vm, o_part;
     int o_T0, o_u0, o_T1, o_z1, o_od, o_ad, o_x1, o_x2, o_w;
+    // Phi-VJP mode only (x is then s [n][D]): seeds on Phi and on grad Phi (NULL: zero), d psi / d s [n][D] or NULL
+    const real* seed_phi;
+    const real* seed_grad;
+    real* grad_s;
 };
 
 template <typename real>
@@ -299,7 +305,11 @@ __device__ __forceinline__ void matvec2(const real* __restrict__ W, int N, int K
     }
 }
 
-template <typename real, int TS, bool WSM>
+// VJP = false: the training step (forward sweep, terminal block, backward sweep of every tile).
+// VJP = true:  the reverse-mode product of Phi.forward / Phi.getGrad (noc_phi_vjp) — the terminal block's two sweeps on one
+//              evaluation per row s_i, with gbar = seed_grad_i and beta = seed_phi_i read from memory, so that sbar is
+//              d psi_i / d s_i and the parameter reductions sum d psi_i / d theta for psi_i = a_i Phi(s_i) + B_i . grad Phi(s_i).
+template <typename real, int TS, bool WSM, bool VJP>
 __global__ void __launch_bounds__(512, 1) rollout_grad_kernel(const GradArgs<real> A) {
     extern __shared__ __align__(16) unsigned char grad_smem[];
     real* sm = reinterpret_cast<real*>(grad_smem);
@@ -656,6 +666,29 @@ __global__ void __launch_bounds__(512, 1) rollout_grad_kernel(const GradArgs<rea
         __syncthreads();
     };
 
+    if constexpr (VJP) {
+        for (int tile = blockIdx.x; tile < A.ntiles; tile += gridDim.x) {
+            const long long base = (long long)tile * TS;
+            for (int i = tid; i < D * TS; i += NT) {
+                const int c = i / TS, si = i % TS;
+                const bool valid = base + si < A.n;
+                const long long row = valid ? base + si : A.n - 1;          // pad rows repeat the last row with zero seeds
+                s[i] = A.x[row * D + c];
+                gb[i] = (valid && A.seed_grad) ? A.seed_grad[row * D + c] : real(0);
+            }
+            if (tid < TS) bt[tid] = (base + tid < A.n && A.seed_phi) ? A.seed_phi[base + tid] : real(0);
+            __syncthreads();
+            primal(true);
+            second_order(true);
+            if (A.grad_s)
+                for (int i = tid; i < D * TS; i += NT) {
+                    const int c = i / TS, si = i % TS;
+                    if (base + si < A.n) A.grad_s[(base + si) * D + c] = sb[i];
+                }
+        }
+        return;
+    }
+
     auto rate = [&](int row, int si) __attribute__((always_inline)) -> real {         // dx/dt = -grad_p H
         if (pr.kind != 2) return -g[row * TS + si];
         if (row < 6) return s[(6 + row) * TS + si];
@@ -789,11 +822,20 @@ __global__ void __launch_bounds__(512, 1) rollout_grad_kernel(const GradArgs<rea
     }
 }
 
+// Tile planning and launch, shared by the training step and the Phi VJP: the packed-weight blob, the gradient sections, the tile
+// width and the shared-memory layout are the same in both modes.
 template <typename real>
-int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const ProbPack& pr, const real* x, long long n,
-                 const double* dtimes, int nt, const double* alph, double t_end, double* out_sums, real* grad, real* grad_x,
-                 int smem_limit, cudaStream_t st) {
+struct GradLaunch {
     GradArgs<real> A;
+    GradSections GS;
+    int TS, NT;
+    size_t smem;
+    bool wsm;
+};
+
+template <typename real>
+static int grad_plan(const char* who, int d, int m, int r, double h, long long n, int smem_limit, GradLaunch<real>& G) {
+    GradArgs<real>& A = G.A;
     memset(&A, 0, sizeof A);
     GradPack<real>& P = A.phi;
     const int D = d + 1;
@@ -804,14 +846,14 @@ int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const P
     P.off_b0 = take(m); P.off_b1 = take(m); P.off_w = take(m); P.off_cw = take(D); P.off_cb = take(1); P.off_A = take(r * D);
     P.blob_len = off;
     // the kernel accumulates into a buffer whose sections start on 16-byte boundaries; unpack_grad_kernel compacts it
-    GradSections GS;
+    GradSections& GS = G.GS;
     int go = 0, co = 0, gi = 0;
     auto gtake = [&](int cnt) { int o = go; GS.src[gi] = go; GS.dst[gi] = co; GS.len[gi] = cnt; ++gi; go += align_up(cnt, 4); co += cnt; return o; };
     P.g_A = gtake(r * D); P.g_cw = gtake(D); P.g_cb = gtake(1); P.g_w = gtake(m); P.g_K0 = gtake(m * D); P.g_b0 = gtake(m);
     P.g_K1 = gtake(m * m); P.g_b1 = gtake(m); P.g_len = go;
 
     const int NT = std::min(512, std::max(32, align_up(std::max(m, D), 32)));
-    if (m > 2048 || (m & 1)) return fail(NOC_ERR_UNSUPPORTED, "noc_ocflow_grad: m = %d (even widths up to 2048)", m);
+    if (m > 2048 || (m & 1)) return fail(NOC_ERR_UNSUPPORTED, "%s: m = %d (even widths up to 2048)", who, m);
     auto plan = [&](int TS, size_t& vec_bytes, bool& wsm) -> size_t {
         int so = 0;
         auto stake = [&](int cnt) { int o = so; so += align_up(cnt, 8); return o; };
@@ -841,15 +883,28 @@ int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const P
     // swap2 1.55 -> 1.41, softcorridor 1.77 -> 1.71; tiles of 1 are slower again: 3.9 / 1.8 / 2.5 ms)
     if (TS == 4 && m <= 64 && wsm && (n + 3) / 4 < 8LL * sm_count()) { TS = 2; smem = plan(TS, vec_bytes, wsm); }
     if (const char* e = getenv("NOC_GRAD_TS")) { int t = atoi(e); if (t == 2 || t == 4 || t == 8) { TS = t; smem = plan(TS, vec_bytes, wsm); } }
-    if (TS < 4 && !wsm) return fail(NOC_ERR_UNSUPPORTED, "noc_ocflow_grad: tiles of %d samples are built for staged weights only", TS);
+    if (TS < 4 && !wsm) return fail(NOC_ERR_UNSUPPORTED, "%s: tiles of %d samples are built for staged weights only", who, TS);
     if (vec_bytes > (size_t)smem_limit)
-        return fail(NOC_ERR_NOMEM, "noc_ocflow_grad: panels of d=%d, m=%d need %zu B of shared memory (> %d)", d, m, vec_bytes, smem_limit);
+        return fail(NOC_ERR_NOMEM, "%s: panels of d=%d, m=%d need %zu B of shared memory (> %d)", who, d, m, vec_bytes, smem_limit);
     A.ntiles = (int)((n + TS - 1) / TS);
     if (getenv("NOC_DEBUG"))
-        fprintf(stderr, "[noc] grad kernel: n=%lld d=%d m=%d TS=%d NT=%d tiles=%d smem=%zu (panels %zu, weights %s) limit=%d\n", n, d, m, TS, NT,
-                A.ntiles, smem, vec_bytes, wsm ? "staged" : "L2", smem_limit);
+        fprintf(stderr, "[noc] %s kernel: n=%lld d=%d m=%d TS=%d NT=%d tiles=%d smem=%zu (panels %zu, weights %s) limit=%d\n", who, n, d, m,
+                TS, NT, A.ntiles, smem, vec_bytes, wsm ? "staged" : "L2", smem_limit);
+    A.use_v4 = wsm ? 0 : 1; A.deep = 1;
+    if (const char* e = getenv("NOC_GRAD_V4")) A.use_v4 = atoi(e);
+    if (const char* e = getenv("NOC_GRAD_DEEP")) A.deep = atoi(e);
+    G.TS = TS; G.NT = NT; G.smem = smem; G.wsm = wsm;
+    return NOC_OK;
+}
 
-    ScratchBuf b_blob, b_xsave, b_partials, b_gacc;       // freed (stream-ordered) on every exit path
+// weight packing, the kernel of the mode (training: nt RK4 steps per tile; VJP: one evaluation per row) and the compaction of the
+// summed parameter gradient into `grad` (NULL: the sums are not wanted)
+template <typename real, bool VJP>
+static int grad_launch(GradLaunch<real>& G, const PhiRaw<real>& raw, real* grad, int nt, cudaStream_t st) {
+    GradArgs<real>& A = G.A;
+    GradPack<real>& P = A.phi;
+    const int m = P.m, D = P.D, d = P.d, TS = G.TS;
+    ScratchBuf b_blob, b_xsave, b_gacc;                    // freed (stream-ordered) on every exit path
     NOC_CUDA(b_blob.alloc(sizeof(real) * (size_t)P.blob_len, st));
     real* blob = b_blob.as<real>();
     NOC_CUDA(cudaMemsetAsync(blob, 0, sizeof(real) * (size_t)P.blob_len, st));
@@ -857,45 +912,76 @@ int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const P
     pack_phi_grad_kernel<real><<<pgrid, 256, 0, st>>>(raw, P, blob);
     count_launch();
     P.blob = blob;
-    NOC_CUDA(b_partials.alloc(sizeof(double) * 8 * (size_t)A.ntiles, st));
     NOC_CUDA(b_gacc.alloc(sizeof(real) * (size_t)P.g_len, st));
     real* gacc = b_gacc.as<real>();
     NOC_CUDA(cudaMemsetAsync(gacc, 0, sizeof(real) * (size_t)P.g_len, st));
+    A.grad = gacc;
+    void (*kern)(const GradArgs<real>) = nullptr;
+    if (TS == 8) kern = G.wsm ? rollout_grad_kernel<real, 8, true, VJP> : rollout_grad_kernel<real, 8, false, VJP>;
+    else if (TS == 4) kern = G.wsm ? rollout_grad_kernel<real, 4, true, VJP> : rollout_grad_kernel<real, 4, false, VJP>;
+    else kern = rollout_grad_kernel<real, 2, true, VJP>;
+    NOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)G.smem));
+    int per_sm = 0;
+    NOC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, G.NT, G.smem));
+    if (per_sm < 1) return fail(NOC_ERR_NOMEM, "%s: kernel does not fit on an SM (%zu B shared memory)", VJP ? "noc_phi_vjp" : "noc_ocflow_grad", G.smem);
+    const int grid = std::max(1, std::min(A.ntiles, per_sm * sm_count()));
+    if (!VJP) {
+        NOC_CUDA(b_xsave.alloc(sizeof(real) * (size_t)grid * nt * 4 * d * TS, st));
+        A.xsave = b_xsave.as<real>();
+    }
+    kern<<<grid, G.NT, G.smem, st>>>(A);
+    count_launch();
+    NOC_CUDA(cudaGetLastError());
+    if (grad) {
+        unpack_grad_kernel<real><<<std::min(std::max(1, ceil_div(P.g_len, 256)), 4 * sm_count()), 256, 0, st>>>(gacc, grad, G.GS);
+        count_launch();
+        NOC_CUDA(cudaGetLastError());
+    }
+    return NOC_OK;
+}
+
+template <typename real>
+int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const ProbPack& pr, const real* x, long long n,
+                 const double* dtimes, int nt, const double* alph, double t_end, double* out_sums, real* grad, real* grad_x,
+                 int smem_limit, cudaStream_t st) {
+    GradLaunch<real> G;
+    int rc = grad_plan<real>("noc_ocflow_grad", d, m, r, h, n, smem_limit, G);
+    if (rc) return rc;
+    GradArgs<real>& A = G.A;
+    ScratchBuf b_partials;                                 // freed (stream-ordered) on every exit path
+    NOC_CUDA(b_partials.alloc(sizeof(double) * 8 * (size_t)A.ntiles, st));
     A.prob = pr; A.x = x; A.n = n; A.nt = nt; A.times = dtimes;
     A.alph0 = (real)alph[0]; A.alph3 = (real)alph[3]; A.alph4 = (real)alph[4]; A.alph5 = (real)alph[5];
     A.t_end = (real)t_end;
-    A.use_v4 = wsm ? 0 : 1; A.deep = 1;
-    if (const char* e = getenv("NOC_GRAD_V4")) A.use_v4 = atoi(e);
-    if (const char* e = getenv("NOC_GRAD_DEEP")) A.deep = atoi(e);
-    A.partials = b_partials.as<double>(); A.grad = gacc; A.grad_x = grad_x;
-    void (*kern)(const GradArgs<real>) = nullptr;
-    if (TS == 8) kern = wsm ? rollout_grad_kernel<real, 8, true> : rollout_grad_kernel<real, 8, false>;
-    else if (TS == 4) kern = wsm ? rollout_grad_kernel<real, 4, true> : rollout_grad_kernel<real, 4, false>;
-    else kern = rollout_grad_kernel<real, 2, true>;
-    NOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-    int per_sm = 0;
-    NOC_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, kern, NT, smem));
-    if (per_sm < 1) return fail(NOC_ERR_NOMEM, "noc_ocflow_grad: kernel does not fit on an SM (%zu B shared memory)", smem);
-    const int grid = std::max(1, std::min(A.ntiles, per_sm * sm_count()));
-    NOC_CUDA(b_xsave.alloc(sizeof(real) * (size_t)grid * nt * 4 * d * TS, st));
-    A.xsave = b_xsave.as<real>();
-    kern<<<grid, NT, smem, st>>>(A);
-    count_launch();
-    NOC_CUDA(cudaGetLastError());
-    unpack_grad_kernel<real><<<std::min(std::max(1, ceil_div(P.g_len, 256)), 4 * sm_count()), 256, 0, st>>>(gacc, grad, GS);
-    count_launch();
-    NOC_CUDA(cudaGetLastError());
+    A.partials = b_partials.as<double>(); A.grad_x = grad_x;
+    rc = grad_launch<real, false>(G, raw, grad, nt, st);
+    if (rc) return rc;
     return launch_finish(A.partials, A.ntiles, out_sums, st);
+}
+
+template <typename real>
+int phi_vjp(int d, int m, int r, double h, const PhiRaw<real>& raw, const real* s, long long n, const real* seed_phi,
+            const real* seed_grad, real* grad, real* grad_s, int smem_limit, cudaStream_t st) {
+    GradLaunch<real> G;
+    int rc = grad_plan<real>("noc_phi_vjp", d, m, r, h, n, smem_limit, G);
+    if (rc) return rc;
+    GradArgs<real>& A = G.A;
+    A.x = s; A.n = n; A.seed_phi = seed_phi; A.seed_grad = seed_grad; A.grad_s = grad_s;
+    return grad_launch<real, true>(G, raw, grad, 0, st);
 }
 
 // one object per precision (Makefile: -DNOC_GRAD_ONLY=32 / 64) so that the two sets of instantiations compile in parallel
 #if !defined(NOC_GRAD_ONLY) || NOC_GRAD_ONLY == 32
 template int grad_rollout<float>(int, int, int, double, const PhiRaw<float>&, const ProbPack&, const float*, long long, const double*, int,
                                  const double*, double, double*, float*, float*, int, cudaStream_t);
+template int phi_vjp<float>(int, int, int, double, const PhiRaw<float>&, const float*, long long, const float*, const float*, float*, float*,
+                            int, cudaStream_t);
 #endif
 #if !defined(NOC_GRAD_ONLY) || NOC_GRAD_ONLY == 64
 template int grad_rollout<double>(int, int, int, double, const PhiRaw<double>&, const ProbPack&, const double*, long long, const double*, int,
                                   const double*, double, double*, double*, double*, int, cudaStream_t);
+template int phi_vjp<double>(int, int, int, double, const PhiRaw<double>&, const double*, long long, const double*, const double*, double*,
+                             double*, int, cudaStream_t);
 #endif
 
 }  // namespace noc

@@ -70,6 +70,11 @@ int grad_rollout(int d, int m, int r, double h, const PhiRaw<real>& raw, const P
                  const double* dtimes, int nt, const double* alph, double t_end, double* out_sums, real* grad, real* grad_x,
                  int smem_limit, cudaStream_t st);
 
+// reverse-mode product of Phi and grad Phi (noc_grad.cu, the training kernel's terminal-block sweeps on one evaluation per row)
+template <typename real>
+int phi_vjp(int d, int m, int r, double h, const PhiRaw<real>& raw, const real* s, long long n, const real* seed_phi,
+            const real* seed_grad, real* grad, real* grad_s, int smem_limit, cudaStream_t st);
+
 // baseline objective (noc_baseline.cu): one warp per sample
 template <typename real>
 int baseline_loss(const ProbPack& pr, const real* U, const real* z0, long long n, int d, int nt, double alphG, real* loss, real* gradU,

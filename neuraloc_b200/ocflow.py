@@ -14,6 +14,9 @@ Deviations from the reference (documented in DESIGN.md):
     with stepper 'rk4' and nTh = 2 runs the fused rollout + discrete-adjoint kernel (noc_ocflow_grad) and `Jc.backward()` works;
     the gradient flows through Jc only (the entries of cs are detached).  Every other combination raises instead of silently
     returning a non-differentiable result;
+  * Phi.forward / Phi.getGrad (phi_apply): with autograd enabled and s or a parameter requiring grad, nTh = 2 nets are
+    differentiated by one noc_phi_vjp call per backward; other depths raise.  The problem evaluators (prob_eval, behind
+    calcLHQW / calcGradpH / calcCtrls and ocOdefun) are forward-only and raise when asked for a gradient;
   * errors raise (ValueError / RuntimeError) instead of print + exit(1).
 """
 import ctypes as C
@@ -148,16 +151,20 @@ def ocflow_grad_sums(x, Phi, prob, tspan, nt, alph=(1.0,) * 6, want_xgrad=False)
         tab = stage_times(float(tspan[0]), float(tspan[1]), nt)
         al = (C.c_double * 6)(*[float(a) for a in alph])
         xin = x.detach().to(device).contiguous()
-        D, m, r = d + 1, phi.m, phi.r
-        P = r * D + D + 1 + m + m * D + m + m * m + m
         sums = torch.empty(8, dtype=torch.float64, device=device)
-        grad = torch.empty(P, dtype=x.dtype, device=device)
+        grad = torch.empty(_grad_len(phi), dtype=x.dtype, device=device)
         gx = torch.empty(n, d, dtype=x.dtype, device=device) if want_xgrad else None
         rc = L.noc_ocflow_grad(C.byref(phi), C.byref(pst), xin.data_ptr(), n, tab, float(tspan[0]), float(tspan[1]), nt, al, code,
                                sums.data_ptr(), grad.data_ptr(), None if gx is None else gx.data_ptr(),
                                torch.cuda.current_stream(device).cuda_stream)
         _cabi.check(rc)
     return sums, grad, gx
+
+
+def _grad_len(phi):
+    """P, the length of the flat parameter gradient of noc_ocflow_grad / noc_phi_vjp for a noc_phi_t with nTh = 2."""
+    D, m, r = phi.d + 1, phi.m, phi.r
+    return r * D + D + 1 + m + m * D + m + m * m + m
 
 
 def split_param_grads(Phi, grad):
@@ -298,8 +305,76 @@ def phi_eval(Phi, s, want_phi=True, want_grad=True):
     return back(op), back(og)
 
 
+def phi_vjp(Phi, s, seed_phi=None, seed_grad=None, want_params=True, want_s=True):
+    """Reverse-mode product of Phi.forward / Phi.getGrad through noc_phi_vjp.  For psi_i = a_i Phi(s_i) + B_i . grad Phi(s_i), with
+    a = seed_phi ([n] or [n,1]) and B = seed_grad ([n, d+1]), None meaning zero, returns on the CUDA device in s.dtype
+    grad_params [P]    SUMS over the rows of d psi_i / d parameter, flat in split_param_grads' order (None unless want_params),
+    grad_s [n, d+1]    d psi_i / d s_i = a_i grad Phi(s_i) + Hess Phi(s_i) B_i (None unless want_s).  nTh = 2 only."""
+    _require_cuda()
+    L = _cabi.lib()
+    code = _dtype_code(s.dtype)
+    device = s.device if s.is_cuda else torch.device("cuda", torch.cuda.current_device())
+    with torch.cuda.device(device):
+        phi = _phi_struct(Phi, device, s.dtype)
+        n, D = s.shape
+        if D != phi.d + 1:
+            raise ValueError("s has %d columns but Phi expects d+1 = %d" % (D, phi.d + 1))
+        if phi.nTh != 2:
+            raise RuntimeError("the reverse-mode product of Phi is implemented for nTh = 2 (got %d)" % phi.nTh)
+        dev = lambda t, shape: None if t is None else t.detach().reshape(shape).to(device=device, dtype=s.dtype).contiguous()
+        sd, a, B = dev(s, (n, D)), dev(seed_phi, (n,)), dev(seed_grad, (n, D))
+        gp = torch.empty(_grad_len(phi), dtype=s.dtype, device=device) if want_params else None
+        gs = torch.empty(n, D, dtype=s.dtype, device=device) if want_s else None
+        ptr = lambda t: None if t is None else t.data_ptr()
+        rc = L.noc_phi_vjp(C.byref(phi), sd.data_ptr(), n, ptr(a), ptr(B), code, ptr(gp), ptr(gs),
+                           torch.cuda.current_stream(device).cuda_stream)
+        _cabi.check(rc)
+    return gp, gs
+
+
+class _PhiWithVJP(torch.autograd.Function):
+    """Phi(s) [n,1] (want_grad False) or grad_s Phi(s) [n, d+1] (want_grad True) by noc_phi_eval — the values of the no-grad
+    path — differentiated with respect to s and every parameter by one noc_phi_vjp call."""
+
+    @staticmethod
+    def forward(ctx, s, Phi, want_grad, *params):
+        out = phi_eval(Phi, s, not want_grad, want_grad)[1 if want_grad else 0]
+        ctx.save_for_backward(s, *params)          # in-place edits of s or of a parameter before backward() raise, as in torch
+        ctx.Phi, ctx.want_grad = Phi, want_grad
+        return out
+
+    @staticmethod
+    @once_differentiable          # the kernel produces first derivatives only: a double backward raises instead of returning zeros
+    def backward(ctx, gout):
+        s, *params = ctx.saved_tensors
+        need_s, need_p = ctx.needs_input_grad[0], ctx.needs_input_grad[3:]
+        gp, gs = phi_vjp(ctx.Phi, s, None if ctx.want_grad else gout, gout if ctx.want_grad else None,
+                         want_params=any(need_p), want_s=need_s)
+        pg = [None] * len(params)
+        if gp is not None:
+            pg = [g.to(device=p.device, dtype=p.dtype) if need else None
+                  for g, p, need in zip(split_param_grads(ctx.Phi, gp), params, need_p)]
+        return (None if gs is None else gs.to(s.device), None, None, *pg)
+
+
+def phi_apply(Phi, s, want_grad):
+    """Phi.forward (want_grad False: [n,1]) or Phi.getGrad (want_grad True: [n, d+1]) on rows s = [x,t].  Differentiable when
+    autograd is enabled and s or a parameter requires grad (nTh = 2); a plain noc_phi_eval call otherwise."""
+    if _wants_grad(s, Phi):
+        nTh = len(Phi.N.layers)
+        if nTh != 2:
+            raise RuntimeError("neuraloc_b200: Phi.forward / Phi.getGrad are differentiable for nTh = 2 (this net has nTh = %d); "
+                               "evaluate deeper nets under torch.no_grad()" % nTh)
+        return _PhiWithVJP.apply(s, Phi, want_grad, *_phi_tensors(Phi))
+    return phi_eval(Phi, s, not want_grad, want_grad)[1 if want_grad else 0]
+
+
 def prob_eval(prob, x, p):
-    """(LHQW [n,4], gradpH [n,d], ctrls [n,nCtrl]) through noc_prob_eval."""
+    """(LHQW [n,4], gradpH [n,d], ctrls [n,nCtrl]) through noc_prob_eval.  Forward-only: the results carry no gradient, so a
+    request for one raises."""
+    if torch.is_grad_enabled() and (x.requires_grad or p.requires_grad):
+        raise RuntimeError("neuraloc_b200: calcLHQW / calcGradpH / calcCtrls (and ocOdefun, which calls them) are forward-only — "
+                           "their results would carry no gradient to x or p. Call them under torch.no_grad() or on detached tensors.")
     _require_cuda()
     L = _cabi.lib()
     code = _dtype_code(x.dtype)
@@ -351,7 +426,7 @@ def ocOdefun(x, t, net, prob, alph=None):
     device evaluators (noc_phi_eval, noc_prob_eval); the rollout itself never calls this."""
     d = x.shape[1] - 4
     s = torch.nn.functional.pad(x[:, :d], (0, 1, 0, 0), value=t)
-    g = phi_eval(net, s, False, True)[1]
+    g = phi_apply(net, s, True)
     lhqw, gph, _ = prob_eval(prob, s[:, :d], g[:, :d])
     hj = torch.abs(g[:, d:d + 1] - lhqw[:, 1:2])
     return torch.cat((-gph, lhqw[:, 0:1], hj, lhqw[:, 2:3], lhqw[:, 3:4]), 1)

@@ -5,6 +5,8 @@ N.nTh, alph, m, d`) and state_dict keys (src/Phi.py:77-87, 32-36), so the pretra
 unchanged, and the same initialisation calls in the same order, so `torch.manual_seed(s); Phi(...)`
 yields the reference's random weights.  `forward` and `getGrad` run on the GPU through
 noc_phi_eval (they are device functions of the rollout kernel); there is no torch arithmetic here.
+Under autograd (nTh = 2) both are differentiable with respect to s and the parameters: the backward
+pass is one noc_phi_vjp call.
 """
 import copy
 
@@ -42,14 +44,12 @@ class Phi(nn.Module):
         self.c.weight.data = torch.zeros(self.c.weight.data.shape)
         self.c.bias.data = torch.zeros(self.c.bias.data.shape)
 
-    def _eval(self, x, want_phi, want_grad):
-        from .ocflow import phi_eval
-        return phi_eval(self, x, want_phi, want_grad)
-
     def forward(self, x):
         """Phi(s) for rows s = [x, t] of shape [n, d+1] -> [n, 1]  (src/Phi.py:91-96), on the GPU."""
-        return self._eval(x, True, False)[0]
+        from .ocflow import phi_apply
+        return phi_apply(self, x, False)
 
     def getGrad(self, x):
         """grad_s Phi -> [n, d+1]  (src/Phi.py:99-138), on the GPU."""
-        return self._eval(x, False, True)[1]
+        from .ocflow import phi_apply
+        return phi_apply(self, x, True)
