@@ -1,9 +1,9 @@
 // noc_api.cu — C ABI (include/noc_b200.h) over the rollout kernels.
 //
-// Host-side work per call: pick the path (small batches -> noc_vec.cu, otherwise a tile configuration for
-// (dtype, m, D)), lay out the shared-memory panels, pack the value-network weights into the K-major blob the
-// kernel reads (a tiny kernel, stream-ordered), launch ONE rollout kernel + a 1-block finishing reduction.
-// All scratch is stream-ordered (cudaMallocAsync), so calls on different streams do not interfere.
+// Host-side work per rollout call: validate the inputs into one RolloutCall (noc_launch.cuh), pick the kernel family
+// (choose_path: tensor-core, small-batch or FMA tile kernel) and hand the call to its launcher, which packs the
+// value-network weights for its kernel (a tiny kernel, stream-ordered) and launches ONE rollout kernel + a 1-block
+// finishing reduction.  All scratch is stream-ordered (ScratchBuf), so calls on different streams do not interfere.
 #include <cuda_runtime.h>
 
 #include <algorithm>
@@ -509,13 +509,15 @@ static void stage_times_host(double t0, double t1, int nt, double* tab) {
 }
 
 // ---- tensor-core path (noc_tc_rollout.cuh): fp32, nTh = 2, m <= 128, shapes instantiated in noc_tc_inst.cu
-int launch_tc_0(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_1(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_2(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_3(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_4(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_5(const TcArgs&, int, cudaStream_t, double*);
-int launch_tc_6(const TcArgs&, int, cudaStream_t, double*);
+int launch_tc_0(const RolloutCall<float>&);
+int launch_tc_1(const RolloutCall<float>&);
+int launch_tc_2(const RolloutCall<float>&);
+int launch_tc_3(const RolloutCall<float>&);
+int launch_tc_4(const RolloutCall<float>&);
+int launch_tc_5(const RolloutCall<float>&);
+int launch_tc_6(const RolloutCall<float>&);
+static int (*const kLaunchTc[])(const RolloutCall<float>&) = {launch_tc_0, launch_tc_1, launch_tc_2, launch_tc_3,
+                                                               launch_tc_4, launch_tc_5, launch_tc_6};
 static int tc_shape_id(const noc_phi_t* ph, const noc_prob_t* pb) {
     if (ph->nTh != 2 || ph->m < 1 || ph->m > 128) return -1;
     int shape = -1;
@@ -533,95 +535,63 @@ static int tc_shape_id(const noc_phi_t* ph, const noc_prob_t* pb) {
     if (tc_smem_bytes(mp, KS) + 1024 > (size_t)g_smem_optin) return -1;      // e.g. d = 24 with m = 128: FMA kernels
     return shape;
 }
-static int tc_launch(int shape, int m, int r, double h, const PhiRaw<float>& raw, const ProbPack& pr, const float* x, long long n,
-                     const double* host_times, int nt, int stepper, int mode, const double* alph, double t_end, double* sums, float* a,
-                     float* b, float* c, int lim, cudaStream_t st) {
-    TcArgs A;
-    memset(&A, 0, sizeof A);
-    const int ch = (shape == 0) ? 64 : 16;               // epilogue chunk x threads per sample of the shape (noc_tc_inst.cu)
-    A.m = m; A.mp = align_up(m, ch); A.h = (float)h; A.r = r;
-    A.K0 = raw.K[0]; A.b0 = raw.b[0]; A.K1 = raw.K[1]; A.b1 = raw.b[1]; A.w = raw.w; A.A = raw.A; A.c_w = raw.c_w; A.c_b = raw.c_b;
-    A.prob = pr; A.x = x; A.n = n; A.nt = nt; A.stepper = stepper; A.mode = mode;
-    A.alph0 = (float)alph[0]; A.alph3 = (float)alph[3]; A.alph4 = (float)alph[4]; A.alph5 = (float)alph[5];
-    A.t_end = (float)t_end;
-    A.out_a = a; A.out_b = b; A.out_c = c;
-    std::vector<TcEval> ev;
-    tc_build_evals(host_times, nt, stepper, mode == NOC_MODE_INTERMEDIATES, t_end, ev);
-    TcEval* dev = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&dev, sizeof(TcEval) * ev.size(), st));
-    NOC_CUDA(cudaMemcpyAsync(dev, ev.data(), sizeof(TcEval) * ev.size(), cudaMemcpyHostToDevice, st));   // pageable: staged before return
-    A.evals = dev; A.nevals = (int)ev.size();
-    int rc;
-    switch (shape) {
-        case 0: rc = launch_tc_0(A, lim, st, sums); break;
-        case 1: rc = launch_tc_1(A, lim, st, sums); break;
-        case 2: rc = launch_tc_2(A, lim, st, sums); break;
-        case 3: rc = launch_tc_3(A, lim, st, sums); break;
-        case 4: rc = launch_tc_4(A, lim, st, sums); break;
-        case 5: rc = launch_tc_5(A, lim, st, sums); break;
-        case 6: rc = launch_tc_6(A, lim, st, sums); break;
-        default: rc = fail(NOC_ERR_ARG, "bad tensor-core shape %d", shape);
-    }
-    cudaError_t e = cudaFreeAsync(dev, st);
-    if (rc == NOC_OK && e != cudaSuccess) rc = fail(NOC_ERR_CUDA, "cudaFreeAsync failed: %s", cudaGetErrorString(e));
-    return rc;
-}
-// the tensor-core kernel exists for fp32 only; the fp64 overload is never selected (use_tc is false) but must compile
-static int tc_launch(int, int, int, double, const PhiRaw<double>&, const ProbPack&, const double*, long long, const double*, int, int,
-                     int, const double*, double, double*, double*, double*, double*, int, cudaStream_t) {
-    return fail(NOC_ERR_UNSUPPORTED, "the tensor-core path is fp32 only");
-}
 
 // ---- streamed tensor-core path (noc_ts_rollout.cuh): fp32, nTh = 2, the 50-agent swarm with 128 < m <= 512
-int launch_ts_swarm50(const TsArgs&, const PhiRaw<float>&, int, int, int, cudaStream_t, double*);
+int launch_ts_swarm50(const RolloutCall<float>&);
 static bool ts_shape_ok(const noc_phi_t* ph, const noc_prob_t* pb) {
     return ph->nTh == 2 && pb->kind == NOC_PROB_SWARMTRAJ && pb->agentDim == 3 && pb->nAgents == 50 && ph->d == 150 && ph->m > 128 &&
            ph->m <= 512 && ts_smem_bytes_50() <= (size_t)g_smem_optin && g_cc_major == 10;
 }
-static int ts_launch(int m, int r, double h, const PhiRaw<float>& raw, const ProbPack& pr, const float* x, long long n, int d,
-                     const double* host_times, int nt, int stepper, int mode, const double* alph, double t_end, double* sums, float* a,
-                     float* b, float* c, int lim, cudaStream_t st) {
-    TsArgs A;
-    memset(&A, 0, sizeof A);
-    A.m = m; A.h = (float)h;
-    A.b1 = raw.b[1]; A.w = raw.w; A.c_w = raw.c_w; A.c_b = raw.c_b;
-    A.prob = pr; A.x = x; A.n = n; A.nt = nt; A.mode = mode;
-    A.alph0 = (float)alph[0]; A.alph3 = (float)alph[3]; A.alph4 = (float)alph[4]; A.alph5 = (float)alph[5];
-    A.out_a = a; A.out_b = b; A.out_c = c;
-    A.f_alphQ = (float)pr.alph_Q; A.f_alphW = (float)pr.alph_W; A.f_cut = (float)pr.cutW; A.f_c2 = (float)(2 * pr.r * pr.r);
-    A.hasQ = (pr.obstacle != 0) && (pr.alph_Q > 0.0); A.hasW = (pr.alph_W != 0.0); A.posQ = (pr.alph_Q > 0.0);
-    A.obstacle = pr.obstacle; A.training = pr.training;
-    {
-        const double r = pr.r;                     // SwarmTraj.py:101-119: the boxes inflated by r (train mode)
-        const double t[10] = {2.0 + r, -2.0 - r, 0.5 + r, -0.5 - r, 7.0 + r, 4.0 + r, 2.0 - r, 1.0 + r, -1.0 - r, 4.0 + r};
-        for (int i = 0; i < 10; ++i) A.thr[i] = (float)t[i];
-    }
-    std::vector<TcEval> ev;
-    tc_build_evals(host_times, nt, stepper, mode == NOC_MODE_INTERMEDIATES, t_end, ev);
-    TcEval* dev = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&dev, sizeof(TcEval) * ev.size(), st));
-    NOC_CUDA(cudaMemcpyAsync(dev, ev.data(), sizeof(TcEval) * ev.size(), cudaMemcpyHostToDevice, st));
-    A.evals = dev; A.nevals = (int)ev.size();
-    int rc = launch_ts_swarm50(A, raw, d + 1, r, lim, st, sums);
-    cudaError_t e = cudaFreeAsync(dev, st);
-    if (rc == NOC_OK && e != cudaSuccess) rc = fail(NOC_ERR_CUDA, "cudaFreeAsync failed: %s", cudaGetErrorString(e));
-    return rc;
+
+// The kernel family of a forward rollout (NOC_PATH_*, recorded for noc_last_path); *tc_shape is the tensor-core shape id, or
+// -1 for the streamed swarm50 kernel.  Small batches (n <= NOC_VEC_MAX: 256, or 64 for swarm50, where the CTA-pair kernel is
+// faster beyond that) run one CTA / cluster per sample; the tensor-core kernels take the fp32 shapes they are written for
+// (NOC_TC=0 keeps the FMA kernels); everything else runs the FMA tile kernel.  NOC_FORCE_PATH=tile|vec|tc pins a path (tests).
+template <typename real>
+static int choose_path(const noc_phi_t* ph, const noc_prob_t* pb, long long n, int* tc_shape) {
+    const bool f32 = std::is_same<real, float>::value;
+    *tc_shape = f32 ? tc_shape_id(ph, pb) : -1;
+    const bool ts = f32 && ts_shape_ok(ph, pb);          // never together with a tc shape (SwarmTraj vs Cross2D / Quadcopter)
+    const char* vec_env = getenv("NOC_VEC_MAX");
+    const char* tc_env = getenv("NOC_TC");
+    const char* force = getenv("NOC_FORCE_PATH");
+    const bool force_vec = force && !strcmp(force, "vec"), force_tile = force && !strcmp(force, "tile");
+    const bool force_tc = force && !strcmp(force, "tc");
+    const long long vec_max = vec_env ? atoll(vec_env) : (ts ? 64 : 256);
+    bool use_vec = force_vec || (n <= vec_max && !force_tile);
+    if (std::max(ph->m, ph->d + 4) > 1024) use_vec = false;
+    bool use_tc = false;
+    if (*tc_shape >= 0 || ts)
+        use_tc = force_tc || (!use_vec && !(tc_env && !strcmp(tc_env, "0")) && !force_tile && !force_vec);
+    g_last_path = use_tc ? NOC_PATH_TENSOR : (use_vec ? NOC_PATH_SAMPLE : NOC_PATH_TILE);
+    return g_last_path;
 }
-static int ts_launch(int, int, double, const PhiRaw<double>&, const ProbPack&, const double*, long long, int, const double*, int, int,
-                     int, const double*, double, double*, double*, double*, double*, int, cudaStream_t) {
-    return fail(NOC_ERR_UNSUPPORTED, "the tensor-core path is fp32 only");
+
+// FMA tile kernel: the first configuration whose panels fit (choose), NOC_FORCE_CFG pins one
+template <typename real>
+static int tile_rollout(const RolloutCall<real>& c) {
+    RolloutArgs<real> A;
+    memset(&A, 0, sizeof A);
+    A.phi.d = c.d; A.phi.D = c.d + 1; A.phi.m = c.m; A.phi.nTh = c.nTh; A.phi.r = c.r; A.phi.h = c.h;
+    copy_common(A, c);
+    A.stepper = c.stepper; A.times = c.times; A.t_end = (real)c.t_end;
+    int cfg_id = -1;
+    size_t smem = 0;
+    const int dtype = std::is_same<real, float>::value ? NOC_F32 : NOC_F64;
+    int rc = choose<real>(A, dtype, c.prob.kind, c.prob.nAgents, cfg_id, smem);
+    if (rc) return rc;
+    return dispatch<real>(cfg_id, A, &c.raw, KMODE_ROLLOUT, smem, c.stream, c.out_sums);
 }
 
 template <typename real>
 static int ocflow_impl(const noc_phi_t* ph, const noc_prob_t* pb, const void* x, int64_t n, const double* stage_times,
                        double t0, double t1, int nt, int stepper, const double* alph, int mode, void* out_costs,
-                       void* zFull, void* ctrlFull, cudaStream_t st, int dtype) {
-    RolloutArgs<real> A;
-    memset(&A, 0, sizeof A);
-    PhiRaw<real> R;
-    int rc = fill_phi<real>(ph, A.phi, R);
+                       void* zFull, void* ctrlFull, cudaStream_t st) {
+    RolloutCall<real> c{};
+    PhiPack<real> P;
+    int rc = fill_phi<real>(ph, P, c.raw);
     if (rc) return rc;
-    rc = check_prob(pb, ph->d, A.prob);
+    rc = check_prob(pb, ph->d, c.prob);
     if (rc) return rc;
     if (!x || n < 1) return fail(NOC_ERR_ARG, "x is NULL or n < 1");
     if (nt < 1) return fail(NOC_ERR_ARG, "nt must be >= 1");
@@ -631,88 +601,43 @@ static int ocflow_impl(const noc_phi_t* ph, const noc_prob_t* pb, const void* x,
     if (mode == NOC_MODE_INTERMEDIATES) { if (!zFull || !ctrlFull) return fail(NOC_ERR_ARG, "intermediates mode needs zFull and ctrlFull"); }
     else if (mode == NOC_MODE_MEAN || mode == NOC_MODE_NOMEAN) { if (!out_costs) return fail(NOC_ERR_ARG, "out_costs is NULL"); }
     else return fail(NOC_ERR_ARG, "unknown mode %d", mode);
-
-    // path: small batches run one CTA per sample (noc_vec.cu), everything else the tile kernel.
-    // NOC_VEC_MAX sets the batch-size threshold, NOC_FORCE_PATH=tile|vec pins a path (tests).
     rc = device_facts();
     if (rc) return rc;
-    long long vec_max = 256;
-    if (const char* e = getenv("NOC_VEC_MAX")) vec_max = atoll(e);
-    if (std::is_same<real, float>::value && ts_shape_ok(ph, pb) && !getenv("NOC_VEC_MAX")) vec_max = 64;   // beyond that the CTA-pair kernel is faster
-    bool use_vec = n <= vec_max;
-    if (const char* e = getenv("NOC_FORCE_PATH")) {
-        if (!strcmp(e, "vec")) use_vec = true;
-        else if (!strcmp(e, "tile")) use_vec = false;
-    }
-    if (std::max(ph->m, ph->d + 4) > 1024) use_vec = false;
-    // tensor-core path (noc_tc_rollout.cuh) for the shapes it is written for; NOC_TC=0 turns it off, NOC_FORCE_PATH=tc forces it
-    bool use_tc = false;
-    const int tc_shape = std::is_same<real, float>::value ? tc_shape_id(ph, pb) : -1;
-    if (tc_shape >= 0) {                                  // on by default; NOC_TC=0 keeps the FMA kernels
-        const char* tc = getenv("NOC_TC");
-        const char* fp = getenv("NOC_FORCE_PATH");
-        use_tc = !use_vec && !(tc && !strcmp(tc, "0"));
-        if (fp && !strcmp(fp, "tc")) use_tc = true;
-        if (fp && (!strcmp(fp, "tile") || !strcmp(fp, "vec"))) use_tc = false;
-        if (use_tc) use_vec = false;
-    }
-    // streamed tensor-core kernel for the wide swarm network (same switches)
-    bool use_ts = false;
-    if (!use_tc && std::is_same<real, float>::value && ts_shape_ok(ph, pb)) {
-        const char* tc = getenv("NOC_TC");
-        const char* fp = getenv("NOC_FORCE_PATH");
-        use_ts = !use_vec && !(tc && !strcmp(tc, "0"));
-        if (fp && !strcmp(fp, "tc")) use_ts = true;
-        if (fp && (!strcmp(fp, "tile") || !strcmp(fp, "vec"))) use_ts = false;
-        if (use_ts) use_vec = false;
-    }
-    g_last_path = (use_tc || use_ts) ? NOC_PATH_TENSOR : (use_vec ? NOC_PATH_SAMPLE : NOC_PATH_TILE);
-
-    int cfg_id = -1;
-    size_t smem = 0;
-    if (!use_vec && !use_tc && !use_ts) {
-        rc = choose<real>(A, dtype, pb->kind, pb->nAgents, cfg_id, smem);
-        if (rc) return rc;
-    }
+    int tc_shape = -1;
+    const int path = choose_path<real>(ph, pb, n, &tc_shape);
 
     std::vector<double> tab((size_t)nt * 5);
     if (stage_times) memcpy(tab.data(), stage_times, sizeof(double) * tab.size());
     else stage_times_host(t0, t1, nt, tab.data());
-    double* dtab = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&dtab, sizeof(double) * tab.size(), st));
-    NOC_CUDA(cudaMemcpyAsync(dtab, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, st));
+    ScratchBuf dtab;
+    NOC_CUDA(dtab.alloc(sizeof(double) * tab.size(), st));
+    NOC_CUDA(cudaMemcpyAsync(dtab.p, tab.data(), sizeof(double) * tab.size(), cudaMemcpyHostToDevice, st));
 
-    A.x = (const real*)x; A.n = n; A.nt = nt; A.stepper = stepper; A.mode = mode; A.times = dtab;
-    A.alph0 = (real)alph[0]; A.alph3 = (real)alph[3]; A.alph4 = (real)alph[4]; A.alph5 = (real)alph[5];
-    A.t_end = (real)t1;
-    A.out_a = (mode == NOC_MODE_NOMEAN) ? (real*)out_costs : nullptr;
-    A.out_b = (real*)zFull; A.out_c = (real*)ctrlFull;
-    if (use_ts)
-        rc = ts_launch(ph->m, ph->r, (double)A.phi.h, R, A.prob, (const real*)x, n, ph->d, tab.data(), nt, stepper, mode, alph, t1,
-                       (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr, A.out_a, A.out_b, A.out_c, g_smem_optin, st);
-    else if (use_tc)
-        rc = tc_launch(tc_shape, ph->m, ph->r, (double)A.phi.h, R, A.prob, (const real*)x, n, tab.data(), nt, stepper, mode, alph, t1,
-                       (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr, A.out_a, A.out_b, A.out_c, g_smem_optin, st);
-    else if (use_vec) {
+    c.d = ph->d; c.m = ph->m; c.nTh = ph->nTh; c.r = ph->r; c.h = P.h;
+    c.x = (const real*)x; c.n = n; c.host_times = tab.data(); c.times = dtab.as<double>();
+    c.nt = nt; c.stepper = stepper; c.mode = mode; c.alph = alph; c.t_end = t1;
+    c.out_sums = (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr;
+    c.out_nomean = (mode == NOC_MODE_NOMEAN) ? (real*)out_costs : nullptr;
+    c.zFull = (real*)zFull; c.ctrlFull = (real*)ctrlFull;
+    c.smem_limit = g_smem_optin; c.stream = st;
+    if (path == NOC_PATH_TENSOR) {
+        if constexpr (std::is_same<real, float>::value) rc = (tc_shape >= 0) ? kLaunchTc[tc_shape](c) : launch_ts_swarm50(c);
+        else rc = fail(NOC_ERR_UNSUPPORTED, "the tensor-core kernels are fp32 only");      // choose_path does not pick them
+    } else if (path == NOC_PATH_SAMPLE) {
         bool took = false;
-        rc = lat_rollout<real>(&took, ph->d, ph->m, ph->nTh, ph->r, (double)A.phi.h, R, A.prob, (const real*)x, n, dtab, nt, stepper, mode,
-                               alph, t1, (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr, A.out_a, A.out_b, A.out_c, g_smem_optin, st);
-        if (rc == NOC_OK && !took)
-        rc = vec_rollout<real>(ph->d, ph->m, ph->nTh, ph->r, (double)A.phi.h, R, A.prob, (const real*)x, n, dtab, nt, stepper, mode, alph,
-                               t1, (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr, A.out_a, A.out_b, A.out_c,
-                               g_smem_optin, st);
+        rc = lat_rollout<real>(c, &took);
+        if (rc == NOC_OK && !took) rc = vec_rollout<real>(c);
     } else
-        rc = dispatch<real>(cfg_id, A, &R, KMODE_ROLLOUT, smem, st, (mode == NOC_MODE_MEAN) ? (double*)out_costs : nullptr);
-    cudaError_t e = cudaFreeAsync(dtab, st);
+        rc = tile_rollout<real>(c);
     if (rc) return rc;
-    if (e != cudaSuccess) return fail(NOC_ERR_CUDA, "cudaFreeAsync failed: %s", cudaGetErrorString(e));
+    NOC_CUDA(dtab.free());
     return NOC_OK;
 }
 
 template <typename real>
 static int ocflow_host_impl(const noc_phi_t* ph, const noc_prob_t* pb, const void* xh, int64_t n, const double* stage_times,
                             double t0, double t1, int nt, int stepper, const double* alph, int mode, void* out_h,
-                            void* z_h, void* c_h, cudaStream_t st, int dtype) {
+                            void* z_h, void* c_h, cudaStream_t st) {
     if (!ph || !pb) return fail(NOC_ERR_ARG, "phi / prob is NULL");
     if (!xh || n < 1) return fail(NOC_ERR_ARG, "x is NULL or n < 1");
     const int d = ph->d;
@@ -736,81 +661,71 @@ static int ocflow_host_impl(const noc_phi_t* ph, const noc_prob_t* pb, const voi
     const long long rows_per = (((n + nchunk - 1) / nchunk + 127) / 128) * 128;
     if (mode == NOC_MODE_MEAN) ob = sizeof(double) * 8 * (size_t)nchunk;
     big_reserve(xb + ob + zb + cb);
-    void *xd = nullptr, *od = nullptr, *zd = nullptr, *cd = nullptr;
-    auto release = [&] {                                   // one cleanup path: every exit frees what was allocated
-        if (xd) cudaFreeAsync(xd, st);
-        if (od) cudaFreeAsync(od, st);
-        if (zd) cudaFreeAsync(zd, st);
-        if (cd) cudaFreeAsync(cd, st);
-        xd = od = zd = cd = nullptr;
-    };
+    int rc = NOC_OK;
+    double sums_h[64 * 8];
     {
-        cudaError_t e = (cudaError_t)big_alloc(&xd, xb, st);
-        if (e == cudaSuccess && ob) e = (cudaError_t)big_alloc(&od, ob, st);
-        if (e == cudaSuccess && zb) e = (cudaError_t)big_alloc(&zd, zb, st);
-        if (e == cudaSuccess && cb) e = (cudaError_t)big_alloc(&cd, cb, st);
+        ScratchBuf xd, od, zd, cd;                         // freed at the end of this block, before the synchronisation below
+        cudaError_t e = xd.alloc_big(xb, st);
+        if (e == cudaSuccess && ob) e = od.alloc_big(ob, st);
+        if (e == cudaSuccess && zb) e = zd.alloc_big(zb, st);
+        if (e == cudaSuccess && cb) e = cd.alloc_big(cb, st);
         if (e != cudaSuccess) {
-            release();
             (void)cudaGetLastError();
             return fail(NOC_ERR_NOMEM, "device buffers for the host entry point (%zu + %zu + %zu + %zu B): %s", xb, ob, zb, cb, cudaGetErrorString(e));
         }
-    }
-    int rc = NOC_OK;
-    double sums_h[64 * 8];
-    if (nchunk == 1) {
-        cudaError_t e = cudaMemcpyAsync(xd, xh, xb, cudaMemcpyHostToDevice, st);
-        if (e != cudaSuccess) { release(); return fail(NOC_ERR_CUDA, "host->device copy failed: %s", cudaGetErrorString(e)); }
-        rc = ocflow_impl<real>(ph, pb, xd, n, stage_times, t0, t1, nt, stepper, alph, mode, od, zd, cd, st, dtype);
-    } else {
-        // streams: `cs` copies; chunks alternate between `st` and `as` so that a chunk's last, partly filled wave of tiles
-        // overlaps the next chunk's first wave instead of idling SMs
-        cudaStream_t cs = nullptr, as = nullptr;
-        cudaEvent_t ready = nullptr, joined = nullptr, copied[64] = {nullptr};
-        // the two helper streams are created once per host thread and device and reused (creating and destroying them per call
-        // showed up as sporadic stalls of the calling thread)
-        static thread_local cudaStream_t t_cs[64] = {nullptr}, t_as[64] = {nullptr};
-        int dev = 0;
-        cudaError_t e = cudaGetDevice(&dev);
-        if (e == cudaSuccess && (dev < 0 || dev >= 64)) e = cudaErrorInvalidDevice;
-        if (e == cudaSuccess && !t_cs[dev]) e = cudaStreamCreateWithFlags(&t_cs[dev], cudaStreamNonBlocking);
-        if (e == cudaSuccess && !t_as[dev]) e = cudaStreamCreateWithFlags(&t_as[dev], cudaStreamNonBlocking);
-        if (e == cudaSuccess) { cs = t_cs[dev]; as = t_as[dev]; }
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ready, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventCreateWithFlags(&joined, cudaEventDisableTiming);
-        if (e == cudaSuccess) e = cudaEventRecord(ready, st);                 // xd / od exist (stream-ordered allocation on st)
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(cs, ready, 0);
-        if (e == cudaSuccess) e = cudaStreamWaitEvent(as, ready, 0);
-        for (int c = 0; c < nchunk && e == cudaSuccess && rc == NOC_OK; ++c) {
-            const long long r0 = (long long)c * rows_per, nr = std::min<long long>(rows_per, n - r0);
-            if (nr <= 0) { nchunk = c; break; }
-            const char* src = (const char*)xh + sizeof(real) * (size_t)r0 * d;
-            char* dst = (char*)xd + sizeof(real) * (size_t)r0 * d;
-            e = cudaMemcpyAsync(dst, src, sizeof(real) * (size_t)nr * d, cudaMemcpyHostToDevice, cs);
-            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&copied[c], cudaEventDisableTiming);
-            if (e == cudaSuccess) e = cudaEventRecord(copied[c], cs);
-            cudaStream_t ks = (c & 1) ? as : st;
-            if (e == cudaSuccess) e = cudaStreamWaitEvent(ks, copied[c], 0);
-            if (e != cudaSuccess) break;
-            void* oc = (mode == NOC_MODE_MEAN) ? (void*)((double*)od + 8 * c) : (void*)((real*)od + 8 * (size_t)r0);
-            rc = ocflow_impl<real>(ph, pb, dst, nr, stage_times, t0, t1, nt, stepper, alph, mode, oc, nullptr, nullptr, ks, dtype);
+        if (nchunk == 1) {
+            e = cudaMemcpyAsync(xd.p, xh, xb, cudaMemcpyHostToDevice, st);
+            if (e != cudaSuccess) return fail(NOC_ERR_CUDA, "host->device copy failed: %s", cudaGetErrorString(e));
+            rc = ocflow_impl<real>(ph, pb, xd.p, n, stage_times, t0, t1, nt, stepper, alph, mode, od.p, zd.p, cd.p, st);
+        } else {
+            // streams: `cs` copies; chunks alternate between `st` and `as` so that a chunk's last, partly filled wave of tiles
+            // overlaps the next chunk's first wave instead of idling SMs
+            cudaStream_t cs = nullptr, as = nullptr;
+            cudaEvent_t ready = nullptr, joined = nullptr, copied[64] = {nullptr};
+            // the two helper streams are created once per host thread and device and reused (creating and destroying them per call
+            // showed up as sporadic stalls of the calling thread)
+            static thread_local cudaStream_t t_cs[64] = {nullptr}, t_as[64] = {nullptr};
+            int dev = 0;
+            e = cudaGetDevice(&dev);
+            if (e == cudaSuccess && (dev < 0 || dev >= 64)) e = cudaErrorInvalidDevice;
+            if (e == cudaSuccess && !t_cs[dev]) e = cudaStreamCreateWithFlags(&t_cs[dev], cudaStreamNonBlocking);
+            if (e == cudaSuccess && !t_as[dev]) e = cudaStreamCreateWithFlags(&t_as[dev], cudaStreamNonBlocking);
+            if (e == cudaSuccess) { cs = t_cs[dev]; as = t_as[dev]; }
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&ready, cudaEventDisableTiming);
+            if (e == cudaSuccess) e = cudaEventCreateWithFlags(&joined, cudaEventDisableTiming);
+            if (e == cudaSuccess) e = cudaEventRecord(ready, st);                 // xd / od exist (stream-ordered allocation on st)
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(cs, ready, 0);
+            if (e == cudaSuccess) e = cudaStreamWaitEvent(as, ready, 0);
+            for (int c = 0; c < nchunk && e == cudaSuccess && rc == NOC_OK; ++c) {
+                const long long r0 = (long long)c * rows_per, nr = std::min<long long>(rows_per, n - r0);
+                if (nr <= 0) { nchunk = c; break; }
+                const char* src = (const char*)xh + sizeof(real) * (size_t)r0 * d;
+                char* dst = xd.as<char>() + sizeof(real) * (size_t)r0 * d;
+                e = cudaMemcpyAsync(dst, src, sizeof(real) * (size_t)nr * d, cudaMemcpyHostToDevice, cs);
+                if (e == cudaSuccess) e = cudaEventCreateWithFlags(&copied[c], cudaEventDisableTiming);
+                if (e == cudaSuccess) e = cudaEventRecord(copied[c], cs);
+                cudaStream_t ks = (c & 1) ? as : st;
+                if (e == cudaSuccess) e = cudaStreamWaitEvent(ks, copied[c], 0);
+                if (e != cudaSuccess) break;
+                void* oc = (mode == NOC_MODE_MEAN) ? (void*)(od.as<double>() + 8 * c) : (void*)(od.as<real>() + 8 * (size_t)r0);
+                rc = ocflow_impl<real>(ph, pb, dst, nr, stage_times, t0, t1, nt, stepper, alph, mode, oc, nullptr, nullptr, ks);
+            }
+            if (e == cudaSuccess && as) e = cudaEventRecord(joined, as);          // st continues after the odd chunks too
+            if (e == cudaSuccess && as) e = cudaStreamWaitEvent(st, joined, 0);
+            if (e != cudaSuccess && rc == NOC_OK) rc = fail(NOC_ERR_CUDA, "chunked host rollout failed: %s", cudaGetErrorString(e));
+            if (cs) cudaStreamSynchronize(cs);
+            if (as) cudaStreamSynchronize(as);
+            for (int c = 0; c < 64; ++c) if (copied[c]) cudaEventDestroy(copied[c]);
+            if (ready) cudaEventDestroy(ready);
+            if (joined) cudaEventDestroy(joined);
         }
-        if (e == cudaSuccess && as) e = cudaEventRecord(joined, as);          // st continues after the odd chunks too
-        if (e == cudaSuccess && as) e = cudaStreamWaitEvent(st, joined, 0);
-        if (e != cudaSuccess && rc == NOC_OK) rc = fail(NOC_ERR_CUDA, "chunked host rollout failed: %s", cudaGetErrorString(e));
-        if (cs) cudaStreamSynchronize(cs);
-        if (as) cudaStreamSynchronize(as);
-        for (int c = 0; c < 64; ++c) if (copied[c]) cudaEventDestroy(copied[c]);
-        if (ready) cudaEventDestroy(ready);
-        if (joined) cudaEventDestroy(joined);
+        if (rc == NOC_OK) {
+            if (ob && out_h) e = cudaMemcpyAsync((mode == NOC_MODE_MEAN) ? (void*)sums_h : out_h, od.p, ob, cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess && zb && z_h) e = cudaMemcpyAsync(z_h, zd.p, zb, cudaMemcpyDeviceToHost, st);
+            if (e == cudaSuccess && cb && c_h) e = cudaMemcpyAsync(c_h, cd.p, cb, cudaMemcpyDeviceToHost, st);
+            if (e != cudaSuccess) rc = fail(NOC_ERR_CUDA, "device->host copy failed: %s", cudaGetErrorString(e));
+        }
     }
-    if (rc == NOC_OK) {
-        cudaError_t e = cudaSuccess;
-        if (ob && out_h) e = cudaMemcpyAsync((mode == NOC_MODE_MEAN) ? (void*)sums_h : out_h, od, ob, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess && zb && z_h) e = cudaMemcpyAsync(z_h, zd, zb, cudaMemcpyDeviceToHost, st);
-        if (e == cudaSuccess && cb && c_h) e = cudaMemcpyAsync(c_h, cd, cb, cudaMemcpyDeviceToHost, st);
-        if (e != cudaSuccess) rc = fail(NOC_ERR_CUDA, "device->host copy failed: %s", cudaGetErrorString(e));
-    }
-    release();
     cudaError_t e = cudaStreamSynchronize(st);
     if (rc == NOC_OK && e != cudaSuccess) rc = fail(NOC_ERR_CUDA, "rollout failed: %s", cudaGetErrorString(e));
     if (rc == NOC_OK && mode == NOC_MODE_MEAN && out_h) {          // chunk partials -> [sums, count], fixed order
@@ -943,9 +858,9 @@ int noc_ocflow(const noc_phi_t* phi, const noc_prob_t* prob, const void* x, int6
                void* zFull, void* ctrlFull, void* stream) {
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == NOC_F32)
-        return ocflow_impl<float>(phi, prob, x, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs, zFull, ctrlFull, st, dtype);
+        return ocflow_impl<float>(phi, prob, x, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs, zFull, ctrlFull, st);
     if (dtype == NOC_F64)
-        return ocflow_impl<double>(phi, prob, x, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs, zFull, ctrlFull, st, dtype);
+        return ocflow_impl<double>(phi, prob, x, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs, zFull, ctrlFull, st);
     return fail(NOC_ERR_ARG, "dtype must be NOC_F32 or NOC_F64");
 }
 
@@ -955,10 +870,10 @@ int noc_ocflow_host(const noc_phi_t* phi, const noc_prob_t* prob, const void* x_
     cudaStream_t st = (cudaStream_t)stream;
     if (dtype == NOC_F32)
         return ocflow_host_impl<float>(phi, prob, x_host, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs_host,
-                                       zFull_host, ctrlFull_host, st, dtype);
+                                       zFull_host, ctrlFull_host, st);
     if (dtype == NOC_F64)
         return ocflow_host_impl<double>(phi, prob, x_host, n, stage_times, t0, t1, nt, stepper, alph, mode, out_costs_host,
-                                        zFull_host, ctrlFull_host, st, dtype);
+                                        zFull_host, ctrlFull_host, st);
     return fail(NOC_ERR_ARG, "dtype must be NOC_F32 or NOC_F64");
 }
 

@@ -432,15 +432,16 @@ static inline int lat_pad(int K, int elt) {       // multiple of 16 bytes, and (
 
 // returns NOC_OK and *took = true when the cluster kernel ran; *took = false means "not applicable, use noc_vec.cu"
 template <typename real>
-int lat_rollout(bool* took, int d, int m, int nTh, int r, double h, const PhiRaw<real>& raw, const ProbPack& pr, const real* x, long long n,
-                const double* dtimes, int nt, int stepper, int mode, const double* alph, double t_end, double* out_sums,
-                real* out_nomean, real* zFull, real* ctrlFull, int smem_limit, cudaStream_t st) {
+int lat_rollout(const RolloutCall<real>& c, bool* took) {
+    const int d = c.d, m = c.m;
+    const long long n = c.n;
+    cudaStream_t st = c.stream;
     *took = false;
-    if (nTh != 2 || d + 4 > 256 || getenv("NOC_NO_LAT")) return NOC_OK;
+    if (c.nTh != 2 || d + 4 > 256 || getenv("NOC_NO_LAT")) return NOC_OK;
     LatArgs<real> A;
     memset(&A, 0, sizeof A);
     const int D = d + 1, elt = (int)sizeof(real);
-    A.d = d; A.D = D; A.m = m; A.r = r; A.h = (real)h;
+    A.d = d; A.D = D; A.m = m; A.r = c.r; A.h = c.h;
     A.Kp_D = lat_pad(D, elt); A.Kp_m = lat_pad(m, elt);
     int NC = 0;
     size_t smem = 0;
@@ -458,10 +459,10 @@ int lat_rollout(bool* took, int d, int m, int nTh, int r, double h, const PhiRaw
         const int mfull = mc * nc, dfull = dc * nc;
         A.o_s = stake(std::max(A.Kp_D, dfull)); A.o_u = stake(std::max(A.Kp_m, mfull)); A.o_y = stake(std::max(A.Kp_m, mfull));
         A.o_v = stake(std::max(A.Kp_m, mfull)); A.o_t = stake(mc); A.o_g = stake(std::max(A.Kp_D, dfull)); A.o_q = stake(std::max(A.Kp_D, dfull));
-        A.o_z0 = stake(d + 4); A.o_za = stake(d + 4); A.o_sc = stake(8); A.o_red = stake(32); A.o_qx = stake(5 * std::max(1, pr.nAgents));
+        A.o_z0 = stake(d + 4); A.o_za = stake(d + 4); A.o_sc = stake(8); A.o_red = stake(32); A.o_qx = stake(5 * std::max(1, c.prob.nAgents));
         A.o_tmp = stake(4 * align_up(std::max(mc, 2 * dc), 8)); A.o_phi = stake(2 * 16); A.o_w = so;      // four exchange slots
         smem = (size_t)(so + A.slice_len) * elt;
-        if (smem > (size_t)smem_limit) return false;
+        if (smem > (size_t)c.smem_limit) return false;
         NC = nc; A.mc = mc; A.dc = dc;
         return true;
     };
@@ -490,37 +491,32 @@ int lat_rollout(bool* took, int d, int m, int nTh, int r, double h, const PhiRaw
         nclusters = (int)std::min<long long>(n, maxc);
         cfg.gridDim = dim3(nclusters * NC);
     }
-    real* blob = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&blob, sizeof(real) * (size_t)A.slice_len * NC, st));
-    lat_pack_kernel<real><<<dim3(std::max(1, std::min(64, ceil_div(A.mc * A.Kp_m, 256))), NC), 256, 0, st>>>(raw, A, blob);
+    ScratchBuf blob, partials;
+    NOC_CUDA(blob.alloc(sizeof(real) * (size_t)A.slice_len * NC, st));
+    lat_pack_kernel<real><<<dim3(std::max(1, std::min(64, ceil_div(A.mc * A.Kp_m, 256))), NC), 256, 0, st>>>(c.raw, A, blob.as<real>());
     count_launch();
-    A.blob = blob;
-    A.prob = pr; A.x = x; A.n = n; A.nt = nt; A.stepper = stepper; A.mode = mode; A.times = dtimes;
-    A.alph0 = (real)alph[0]; A.alph3 = (real)alph[3]; A.alph4 = (real)alph[4]; A.alph5 = (real)alph[5];
-    A.t_end = (real)t_end;
-    A.out_a = out_nomean; A.out_b = zFull; A.out_c = ctrlFull;
-    double* partials = nullptr;
-    if (mode == NOC_MODE_MEAN) {
-        NOC_CUDA(cudaMallocAsync((void**)&partials, sizeof(double) * 8 * (size_t)n, st));
-        A.partials = partials;
+    A.blob = blob.as<real>();
+    copy_common(A, c);
+    A.stepper = c.stepper; A.times = c.times; A.t_end = (real)c.t_end;
+    if (c.mode == NOC_MODE_MEAN) {
+        NOC_CUDA(partials.alloc(sizeof(double) * 8 * (size_t)n, st));
+        A.partials = partials.as<double>();
     }
     if (getenv("NOC_DEBUG")) fprintf(stderr, "[noc] latency kernel: cluster of %d, %d units + %d components per CTA, smem %zu B, %d clusters\n", NC, A.mc, A.dc, smem, nclusters);
     NOC_CUDA(cudaLaunchKernelEx(&cfg, kern, A));
     count_launch();
     NOC_CUDA(cudaGetLastError());
-    if (partials) {
-        int frc = launch_finish(partials, (int)n, out_sums, st);
+    if (partials.p) {
+        int frc = launch_finish(partials.as<double>(), (int)n, c.out_sums, st);
         if (frc) return frc;
-        NOC_CUDA(cudaFreeAsync(partials, st));
+        NOC_CUDA(partials.free());
     }
-    NOC_CUDA(cudaFreeAsync(blob, st));
+    NOC_CUDA(blob.free());
     *took = true;
     return NOC_OK;
 }
 
-template int lat_rollout<float>(bool*, int, int, int, int, double, const PhiRaw<float>&, const ProbPack&, const float*, long long,
-                                const double*, int, int, int, const double*, double, double*, float*, float*, float*, int, cudaStream_t);
-template int lat_rollout<double>(bool*, int, int, int, int, double, const PhiRaw<double>&, const ProbPack&, const double*, long long,
-                                 const double*, int, int, int, const double*, double, double*, double*, double*, double*, int, cudaStream_t);
+template int lat_rollout<float>(const RolloutCall<float>&, bool*);
+template int lat_rollout<double>(const RolloutCall<double>&, bool*);
 
 }  // namespace noc

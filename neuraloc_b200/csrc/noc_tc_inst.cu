@@ -43,7 +43,5 @@ using Shape = TcShape<0, 10, 16, 3>;    // Cross2D, 10 agents, d = 20 (swap12_5p
 
 #define NOC_TC_NAME2(k) launch_tc_##k
 #define NOC_TC_NAME(k) NOC_TC_NAME2(k)
-int NOC_TC_NAME(NOC_TC_SHAPE)(const TcArgs& A, int smem_limit, cudaStream_t st, double* out_sums) {
-    return launch_tc<Shape>(A, smem_limit, st, out_sums);
-}
+int NOC_TC_NAME(NOC_TC_SHAPE)(const RolloutCall<float>& c) { return launch_tc<Shape>(c); }
 }  // namespace noc

@@ -706,6 +706,18 @@ static inline void tc_build_evals(const double* tab, int nt, int stepper, bool i
     ev.push_back(e);
 }
 
+// builds the evaluation sequence of the rollout `c` and uploads it (stream-ordered) into `buf` for A.evals / A.nevals
+template <class Args>
+cudaError_t tc_upload_evals(const RolloutCall<float>& c, Args& A, ScratchBuf& buf) {
+    std::vector<TcEval> ev;
+    tc_build_evals(c.host_times, c.nt, c.stepper, c.mode == NOC_MODE_INTERMEDIATES, c.t_end, ev);
+    A.nevals = (int)ev.size();
+    cudaError_t e = buf.alloc(sizeof(TcEval) * ev.size(), c.stream);
+    if (e == cudaSuccess) e = cudaMemcpyAsync(buf.p, ev.data(), sizeof(TcEval) * ev.size(), cudaMemcpyHostToDevice, c.stream);   // pageable: staged before return
+    A.evals = buf.as<TcEval>();
+    return e;
+}
+
 // staging buffer [tile][step][row][128] -> zFull [n, NZ, ntp1] and ctrlFull [n, NCTRL, ntp1] (last dim contiguous).
 // One block per (tile, row): coalesced 512-byte reads, a padded shared-memory transpose, (nt+1)-float contiguous writes.
 constexpr int kUntileSteps = 64;
@@ -729,7 +741,17 @@ static __global__ void __launch_bounds__(128) tc_untile_kernel(const float* __re
 }
 
 template <class SH>
-int launch_tc(TcArgs A, int smem_limit, cudaStream_t st, double* out_sums) {
+int launch_tc(const RolloutCall<float>& c) {
+    const int smem_limit = c.smem_limit;
+    cudaStream_t st = c.stream;
+    TcArgs A;
+    memset(&A, 0, sizeof A);
+    copy_common(A, c);
+    A.m = c.m; A.mp = align_up(c.m, SH::KIND == 2 ? 64 : 16); A.h = c.h; A.r = c.r;   // mp: as tc_shape_id (noc_api.cu)
+    A.K0 = c.raw.K[0]; A.b0 = c.raw.b[0]; A.K1 = c.raw.K[1]; A.b1 = c.raw.b[1]; A.w = c.raw.w; A.A = c.raw.A; A.c_w = c.raw.c_w; A.c_b = c.raw.c_b;
+    A.stepper = c.stepper; A.t_end = (float)c.t_end;
+    ScratchBuf evals, partials, stage;
+    NOC_CUDA(tc_upload_evals(c, A, evals));
     const size_t smem = tc_smem_bytes(A.mp, SH::KS);
     auto kern = (A.mode == NOC_MODE_INTERMEDIATES) ? rollout_tc_kernel<SH, true> : rollout_tc_kernel<SH, false>;
     if (smem + 1024 > (size_t)smem_limit) return fail(NOC_ERR_NOMEM, "tensor-core rollout needs %zu B of shared memory", smem);
@@ -791,34 +813,33 @@ int launch_tc(TcArgs A, int smem_limit, cudaStream_t st, double* out_sums) {
     if (getenv("NOC_DEBUG"))
         fprintf(stderr, "[noc] tc rollout: mp=%d KS=%d smem=%zu tmem_cols=%d CTAs/SM=%d grid=%d tiles=%d\n", A.mp, SH::KS, smem,
                 A.tmem_cols, per_sm, grid, A.ntiles);
-    double* partials = nullptr;
     if (A.mode == NOC_MODE_MEAN) {
-        NOC_CUDA(cudaMallocAsync((void**)&partials, sizeof(double) * 8 * (size_t)grid, st));
-        A.partials = partials;
+        NOC_CUDA(partials.alloc(sizeof(double) * 8 * (size_t)grid, st));
+        A.partials = partials.as<double>();
     }
     // intermediates: stage the trajectories tile-major (coalesced) and transpose afterwards; if the staging buffer (as large
     // as the outputs) cannot be allocated the kernel writes the reference layout directly (strided, slower, same result)
-    float* stage = nullptr;
     if (A.mode == NOC_MODE_INTERMEDIATES) {
         const size_t bytes = sizeof(float) * (size_t)A.ntiles * (A.nt + 1) * (SH::NZ + SH::NCTRL) * 128;
         big_reserve(bytes);                              // repeated intermediates calls reuse the staging buffer instead of paying the driver
-        if (big_alloc((void**)&stage, bytes, st) != (int)cudaSuccess) { stage = nullptr; (void)cudaGetLastError(); }
+        if (stage.alloc_big(bytes, st) != cudaSuccess) (void)cudaGetLastError();
     }
-    A.stage = stage;
+    A.stage = stage.as<float>();
     kern<<<grid, SH::NT, smem_req, st>>>(A);
     count_launch();
     NOC_CUDA(cudaGetLastError());
-    if (stage) {
-        tc_untile_kernel<<<dim3(A.ntiles, SH::NZ + SH::NCTRL), 128, 0, st>>>(stage, A.out_b, A.out_c, A.n, A.nt + 1, SH::NZ, SH::NCTRL);
+    if (stage.p) {
+        tc_untile_kernel<<<dim3(A.ntiles, SH::NZ + SH::NCTRL), 128, 0, st>>>(A.stage, A.out_b, A.out_c, A.n, A.nt + 1, SH::NZ, SH::NCTRL);
         count_launch();
         NOC_CUDA(cudaGetLastError());
-        NOC_CUDA(cudaFreeAsync(stage, st));
+        NOC_CUDA(stage.free());
     }
-    if (partials) {
-        int frc = launch_finish(partials, grid, out_sums, st);
+    if (partials.p) {
+        int frc = launch_finish(A.partials, grid, c.out_sums, st);
         if (frc) return frc;
-        NOC_CUDA(cudaFreeAsync(partials, st));
+        NOC_CUDA(partials.free());
     }
+    NOC_CUDA(evals.free());
     return NOC_OK;
 }
 

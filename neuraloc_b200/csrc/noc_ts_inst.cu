@@ -2,7 +2,5 @@
 #include "noc_ts_rollout.cuh"
 
 namespace noc {
-int launch_ts_swarm50(const TsArgs& A, const PhiRaw<float>& raw, int D, int r, int smem_limit, cudaStream_t st, double* out_sums) {
-    return launch_ts<TsShape<50>>(A, raw, D, r, smem_limit, st, out_sums);
-}
+int launch_ts_swarm50(const RolloutCall<float>& c) { return launch_ts<TsShape<50>>(c); }
 }  // namespace noc

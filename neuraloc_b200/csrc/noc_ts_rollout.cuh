@@ -940,10 +940,27 @@ static inline ts_encode_fn ts_get_encode() {
 static inline size_t ts_smem_bytes_50() { return (size_t)TsShape<50>::SMEM; }
 
 template <class SH>
-int launch_ts(TsArgs A, const PhiRaw<float>& raw, int D, int r, int smem_limit, cudaStream_t st, double* out_sums) {
+int launch_ts(const RolloutCall<float>& c) {
+    cudaStream_t st = c.stream;
+    const ProbPack& pr = c.prob;
+    TsArgs A;
+    memset(&A, 0, sizeof A);
+    copy_common(A, c);
+    A.m = c.m; A.h = c.h;
+    A.b1 = c.raw.b[1]; A.w = c.raw.w; A.c_w = c.raw.c_w; A.c_b = c.raw.c_b;
+    A.f_alphQ = (float)pr.alph_Q; A.f_alphW = (float)pr.alph_W; A.f_cut = (float)pr.cutW; A.f_c2 = (float)(2 * pr.r * pr.r);
+    A.hasQ = (pr.obstacle != 0) && (pr.alph_Q > 0.0); A.hasW = (pr.alph_W != 0.0); A.posQ = (pr.alph_Q > 0.0);
+    A.obstacle = pr.obstacle; A.training = pr.training;
+    {
+        const double r = pr.r;                     // SwarmTraj.py:101-119: the boxes inflated by r (train mode)
+        const double t[10] = {2.0 + r, -2.0 - r, 0.5 + r, -0.5 - r, 7.0 + r, 4.0 + r, 2.0 - r, 1.0 + r, -1.0 - r, 4.0 + r};
+        for (int i = 0; i < 10; ++i) A.thr[i] = (float)t[i];
+    }
+    ScratchBuf evals, blob, aux, scratch, partials, stage;     // aux: [3] max bits, [6] scales (+ pad)
+    NOC_CUDA(tc_upload_evals(c, A, evals));
     const size_t smem = SH::SMEM;
     auto kern = (A.mode == NOC_MODE_INTERMEDIATES) ? rollout_ts_kernel<SH, true> : rollout_ts_kernel<SH, false>;
-    if (smem > (size_t)smem_limit) return fail(NOC_ERR_NOMEM, "streamed tensor-core rollout needs %zu B of shared memory", smem);
+    if (smem > (size_t)c.smem_limit) return fail(NOC_ERR_NOMEM, "streamed tensor-core rollout needs %zu B of shared memory", smem);
     ts_encode_fn encode = ts_get_encode();
     if (!encode) return fail(NOC_ERR_CUDA, "cuTensorMapEncodeTiled is not available from this driver");
     NOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
@@ -951,19 +968,15 @@ int launch_ts(TsArgs A, const PhiRaw<float>& raw, int D, int r, int smem_limit, 
     const int clusters = std::max(1, std::min(A.ntiles, sm_count() / 2));
     const int grid = 2 * clusters;
     const size_t blob_bytes = (size_t)2 * SH::NSTAGE * SH::STAGE_BYTES;
-    unsigned char* blob = nullptr;
-    float* aux = nullptr;            // [3] max bits, [6] scales (+ pad)
-    float* scratch = nullptr;
-    double* partials = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&blob, blob_bytes, st));
-    NOC_CUDA(cudaMallocAsync((void**)&aux, 64, st));
-    NOC_CUDA(cudaMallocAsync((void**)&scratch, sizeof(float) * (size_t)SH::SCR * grid, st));
-    NOC_CUDA(cudaMemsetAsync(blob, 0, blob_bytes, st));
-    NOC_CUDA(cudaMemsetAsync(aux, 0, 64, st));
+    NOC_CUDA(blob.alloc(blob_bytes, st));
+    NOC_CUDA(aux.alloc(64, st));
+    NOC_CUDA(scratch.alloc(sizeof(float) * (size_t)SH::SCR * grid, st));
+    NOC_CUDA(cudaMemsetAsync(blob.p, 0, blob_bytes, st));
+    NOC_CUDA(cudaMemsetAsync(aux.p, 0, 64, st));
     TsPackArgs P;
-    P.m = A.m; P.D = D; P.r = r;
-    P.K0 = raw.K[0]; P.b0 = raw.b[0]; P.K1 = raw.K[1]; P.A = raw.A; P.c_w = raw.c_w;
-    P.maxbits = reinterpret_cast<unsigned*>(aux); P.scales = aux + 4; P.blob = blob;
+    P.m = A.m; P.D = c.d + 1; P.r = c.r;
+    P.K0 = c.raw.K[0]; P.b0 = c.raw.b[0]; P.K1 = c.raw.K[1]; P.A = c.raw.A; P.c_w = c.raw.c_w;
+    P.maxbits = aux.as<unsigned>(); P.scales = aux.as<float>() + 4; P.blob = blob.as<unsigned char>();
     {
         // The tensor core's fp32 accumulate rounds toward zero: measured -0.137 ulp of the result per accumulating MMA
         // (scripts/tc_bias_probe.py), i.e. a relative shrink of 0.137 * 0.72 * 2^-23 = 1.18e-8 per MMA on average over the
@@ -988,28 +1001,27 @@ int launch_ts(TsArgs A, const PhiRaw<float>& raw, int D, int r, int smem_limit, 
     const cuuint64_t gdim[2] = {64, (cuuint64_t)(blob_bytes / 128)};
     const cuuint64_t gstr[1] = {128};
     const cuuint32_t box[2] = {64, 128}, estr[2] = {1, 1};
-    CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, blob, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
+    CUresult cr = encode(&tmap, CU_TENSOR_MAP_DATA_TYPE_UINT16, 2, blob.p, gdim, gstr, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
                          CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (cr != CUDA_SUCCESS) return fail(NOC_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)cr);
-    A.scales = aux + 4;
-    A.scratch = scratch;
+    A.scales = P.scales;
+    A.scratch = scratch.as<float>();
     if (A.mode == NOC_MODE_MEAN) {
-        NOC_CUDA(cudaMallocAsync((void**)&partials, sizeof(double) * 8 * (size_t)grid, st));
-        NOC_CUDA(cudaMemsetAsync(partials, 0, sizeof(double) * 8 * (size_t)grid, st));
-        A.partials = partials;
+        NOC_CUDA(partials.alloc(sizeof(double) * 8 * (size_t)grid, st));
+        NOC_CUDA(cudaMemsetAsync(partials.p, 0, sizeof(double) * 8 * (size_t)grid, st));
+        A.partials = partials.as<double>();
     }
     if (getenv("NOC_DEBUG"))
         fprintf(stderr, "[noc] ts rollout: smem=%zu grid=%d (clusters of 2) tiles=%d stages/eval=%d evals=%d\n", smem, grid, A.ntiles,
                 SH::NSTAGE, A.nevals);
     // intermediates: stage the trajectories tile-major (coalesced) and transpose afterwards; if the staging buffer (as large as
     // the outputs) cannot be allocated the kernel writes the reference layout directly (strided, slower, same result)
-    float* stage = nullptr;
     if (A.mode == NOC_MODE_INTERMEDIATES && !getenv("NOC_TS_NOSTAGE")) {
         const size_t bytes = sizeof(float) * (size_t)A.ntiles * (A.nt + 1) * (SH::NZ + SH::d) * 128;
         big_reserve(bytes);                              // repeated intermediates calls reuse the staging buffer instead of paying the driver
-        if (big_alloc((void**)&stage, bytes, st) != (int)cudaSuccess) { stage = nullptr; (void)cudaGetLastError(); }
+        if (stage.alloc_big(bytes, st) != cudaSuccess) (void)cudaGetLastError();
     }
-    A.stage = stage;
+    A.stage = stage.as<float>();
     long long* trace = nullptr;
     if (getenv("NOC_TS_TRACE")) {
         NOC_CUDA(cudaMalloc((void**)&trace, sizeof(long long) * 20 * 256 * 2));
@@ -1032,20 +1044,21 @@ int launch_ts(TsArgs A, const PhiRaw<float>& raw, int D, int r, int smem_limit, 
         }
         cudaFree(trace);
     }
-    if (stage) {
-        tc_untile_kernel<<<dim3(A.ntiles, SH::NZ + SH::d), 128, 0, st>>>(stage, A.out_b, A.out_c, A.n, A.nt + 1, SH::NZ, SH::d);
+    if (stage.p) {
+        tc_untile_kernel<<<dim3(A.ntiles, SH::NZ + SH::d), 128, 0, st>>>(A.stage, A.out_b, A.out_c, A.n, A.nt + 1, SH::NZ, SH::d);
         count_launch();
         NOC_CUDA(cudaGetLastError());
-        NOC_CUDA(cudaFreeAsync(stage, st));
+        NOC_CUDA(stage.free());
     }
-    if (partials) {
-        int frc = launch_finish(partials, grid, out_sums, st);
+    if (partials.p) {
+        int frc = launch_finish(A.partials, grid, c.out_sums, st);
         if (frc) return frc;
-        NOC_CUDA(cudaFreeAsync(partials, st));
+        NOC_CUDA(partials.free());
     }
-    NOC_CUDA(cudaFreeAsync(scratch, st));
-    NOC_CUDA(cudaFreeAsync(aux, st));
-    NOC_CUDA(cudaFreeAsync(blob, st));
+    NOC_CUDA(scratch.free());
+    NOC_CUDA(aux.free());
+    NOC_CUDA(blob.free());
+    NOC_CUDA(evals.free());
     return NOC_OK;
 }
 

@@ -349,13 +349,14 @@ __global__ void rollout_vec_kernel(const VecArgs<real> A) {
 }
 
 template <typename real>
-int vec_rollout(int d, int m, int nTh, int r, double h, const PhiRaw<real>& raw, const ProbPack& pr, const real* x, long long n,
-                const double* dtimes, int nt, int stepper, int mode, const double* alph, double t_end, double* out_sums,
-                real* out_nomean, real* zFull, real* ctrlFull, int smem_limit, cudaStream_t st) {
+int vec_rollout(const RolloutCall<real>& c) {
+    const int d = c.d, m = c.m, nTh = c.nTh;
+    const long long n = c.n;
+    cudaStream_t st = c.stream;
     VecArgs<real> A;
     memset(&A, 0, sizeof A);
     VecPack<real>& P = A.phi;
-    P.d = d; P.D = d + 1; P.m = m; P.nTh = nTh; P.r = r; P.h = (real)h;
+    P.d = d; P.D = d + 1; P.m = m; P.nTh = nTh; P.r = c.r; P.h = c.h;
     const int D = d + 1;
     int off = 0;
     auto take = [&](int cnt) { int o = off; off += align_up(cnt, 8); return o; };
@@ -372,26 +373,23 @@ int vec_rollout(int d, int m, int nTh, int r, double h, const PhiRaw<real>& raw,
     const int nthreads = std::min(1024, std::max(32, align_up(std::max(std::max(m, D), d + 4), 32)));
     A.o_s = stake(D); A.o_u = stake(m); A.o_u2 = stake(m); A.o_t = stake(std::max(1, nTh - 1) * m); A.o_zb = stake(m);
     A.o_g = stake(D); A.o_q = stake(D); A.o_z0 = stake(d + 4); A.o_za = stake(d + 4); A.o_sc = stake(8); A.o_red = stake(32);
-    A.o_qx = stake(5 * std::max(1, pr.nAgents)); A.o_w = so;
+    A.o_qx = stake(5 * std::max(1, c.prob.nAgents)); A.o_w = so;
     const size_t vec_bytes = (size_t)so * sizeof(real);
-    const bool wsm = vec_bytes + (size_t)P.blob_len * sizeof(real) <= (size_t)smem_limit;
+    const bool wsm = vec_bytes + (size_t)P.blob_len * sizeof(real) <= (size_t)c.smem_limit;
     const size_t smem = vec_bytes + (wsm ? (size_t)P.blob_len * sizeof(real) : 0);
 
-    real* blob = nullptr;
-    NOC_CUDA(cudaMallocAsync((void**)&blob, sizeof(real) * (size_t)P.blob_len, st));
-    NOC_CUDA(cudaMemsetAsync(blob, 0, sizeof(real) * (size_t)P.blob_len, st));
+    ScratchBuf blob, partials;
+    NOC_CUDA(blob.alloc(sizeof(real) * (size_t)P.blob_len, st));
+    NOC_CUDA(cudaMemsetAsync(blob.p, 0, sizeof(real) * (size_t)P.blob_len, st));
     int pgrid = std::min(std::max(1, ceil_div(std::max(m * m, m * D), 256)), 4 * sm_count());
-    pack_phi_plain_kernel<real><<<pgrid, 256, 0, st>>>(raw, P, blob);
+    pack_phi_plain_kernel<real><<<pgrid, 256, 0, st>>>(c.raw, P, blob.as<real>());
     count_launch();
-    P.blob = blob;
-    A.prob = pr; A.x = x; A.n = n; A.nt = nt; A.stepper = stepper; A.mode = mode; A.times = dtimes;
-    A.alph0 = (real)alph[0]; A.alph3 = (real)alph[3]; A.alph4 = (real)alph[4]; A.alph5 = (real)alph[5];
-    A.t_end = (real)t_end;
-    A.out_a = out_nomean; A.out_b = zFull; A.out_c = ctrlFull;
-    double* partials = nullptr;
-    if (mode == NOC_MODE_MEAN) {
-        NOC_CUDA(cudaMallocAsync((void**)&partials, sizeof(double) * 8 * (size_t)n, st));
-        A.partials = partials;
+    P.blob = blob.as<real>();
+    copy_common(A, c);
+    A.stepper = c.stepper; A.times = c.times; A.t_end = (real)c.t_end;
+    if (c.mode == NOC_MODE_MEAN) {
+        NOC_CUDA(partials.alloc(sizeof(double) * 8 * (size_t)n, st));
+        A.partials = partials.as<double>();
     }
     const bool onewarp = wsm && nthreads == 32;
     auto kern = onewarp ? rollout_vec_kernel<real, true, true>
@@ -401,18 +399,16 @@ int vec_rollout(int d, int m, int nTh, int r, double h, const PhiRaw<real>& raw,
     kern<<<grid, nthreads, smem, st>>>(A);
     count_launch();
     NOC_CUDA(cudaGetLastError());
-    if (partials) {
-        int frc = launch_finish(partials, (int)n, out_sums, st);
+    if (partials.p) {
+        int frc = launch_finish(partials.as<double>(), (int)n, c.out_sums, st);
         if (frc) return frc;
-        NOC_CUDA(cudaFreeAsync(partials, st));
+        NOC_CUDA(partials.free());
     }
-    NOC_CUDA(cudaFreeAsync(blob, st));
+    NOC_CUDA(blob.free());
     return NOC_OK;
 }
 
-template int vec_rollout<float>(int, int, int, int, double, const PhiRaw<float>&, const ProbPack&, const float*, long long,
-                                const double*, int, int, int, const double*, double, double*, float*, float*, float*, int, cudaStream_t);
-template int vec_rollout<double>(int, int, int, int, double, const PhiRaw<double>&, const ProbPack&, const double*, long long,
-                                 const double*, int, int, int, const double*, double, double*, double*, double*, double*, int, cudaStream_t);
+template int vec_rollout<float>(const RolloutCall<float>&);
+template int vec_rollout<double>(const RolloutCall<double>&);
 
 }  // namespace noc

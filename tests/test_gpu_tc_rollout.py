@@ -178,7 +178,26 @@ def test_path_selection(nb, monkeypatch):
         monkeypatch.delenv("NOC_TC")
         nb.OCflow(x.double(), net.double(), product_setup("swap12", torch.float64)[1], [0.0, 1.0], 4, "rk4", meta["alph"])
         assert nb._cabi.last_path() == "tile"                      # fp64 has no tensor-core kernel
+        for n, env, want in [(8, {"NOC_FORCE_PATH": "tc"}, "tensor"),
+                             (1000, {"NOC_TC": "0", "NOC_FORCE_PATH": "tc"}, "tensor"),      # forcing wins over NOC_TC=0
+                             (1000, {"NOC_FORCE_PATH": "vec"}, "sample"),
+                             (8, {"NOC_FORCE_PATH": "tile"}, "tile")]:
+            for k, v in env.items():
+                monkeypatch.setenv(k, v)
+            nb.OCflow(x[:n].contiguous(), net, prob, [0.0, 1.0], 4, "rk4", meta["alph"])
+            assert nb._cabi.last_path() == want, (n, env)
+            for k in env:
+                monkeypatch.delenv(k)
         net5, prob5, xinit5, meta5 = product_setup("swarm50", torch.float32)
+        for n, env, want in [(100, {}, "tensor"),                       # swarm50's small-batch threshold is 64, not 256
+                             (64, {}, "sample"),
+                             (100, {"NOC_VEC_MAX": "256"}, "sample")]:   # an explicit threshold replaces the 64
+            for k, v in env.items():
+                monkeypatch.setenv(k, v)
+            nb.OCflow(xinit5.repeat(n, 1), net5, prob5, [0.0, 1.0], 4, "rk4", meta5["alph"])
+            assert nb._cabi.last_path() == want, (n, env)
+            for k in env:
+                monkeypatch.delenv(k)
         Jc, cs = nb.OCflow(xinit5.repeat(300, 1), net5, prob5, [0.0, 1.0], 4, "rk4", meta5["alph"])
         assert nb._cabi.last_path() == "tensor" and np.isfinite(float(Jc))      # the streamed CTA-pair kernel (m = 512)
         monkeypatch.setenv("NOC_TC", "0")
