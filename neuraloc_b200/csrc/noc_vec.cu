@@ -106,7 +106,7 @@ __device__ __forceinline__ real gemv_col(const real* __restrict__ W, int N, cons
 }
 
 template <typename real, bool WSM, bool ONEWARP>
-__global__ void rollout_vec_kernel(const VecArgs<real> A) {
+__device__ __forceinline__ void rollout_vec_body(const VecArgs<real>& A) {
     extern __shared__ __align__(16) unsigned char vec_smem[];
     real* sm = reinterpret_cast<real*>(vec_smem);
     const int tid = threadIdx.x, NT = blockDim.x;
@@ -348,6 +348,15 @@ __global__ void rollout_vec_kernel(const VecArgs<real> A) {
     }
 }
 
+template <typename real, bool WSM, bool ONEWARP>
+__global__ void rollout_vec_kernel(const VecArgs<real> A) { rollout_vec_body<real, WSM, ONEWARP>(A); }
+
+// The same kernel built for 1024 threads per block (at most 64 registers per thread).  Left to itself the compiler gives the
+// fp64 kernels 96-116 registers, which leaves room for 544-672 threads per block, not for the 1024 that m up to 1024 needs:
+// vec_rollout takes this copy for exactly the blocks the other one cannot launch.
+template <typename real, bool WSM>
+__global__ void __launch_bounds__(1024) rollout_vec_kernel_1024(const VecArgs<real> A) { rollout_vec_body<real, WSM, false>(A); }
+
 template <typename real>
 int vec_rollout(const RolloutCall<real>& c) {
     const int d = c.d, m = c.m, nTh = c.nTh;
@@ -394,6 +403,10 @@ int vec_rollout(const RolloutCall<real>& c) {
     const bool onewarp = wsm && nthreads == 32;
     auto kern = onewarp ? rollout_vec_kernel<real, true, true>
                         : (wsm ? rollout_vec_kernel<real, true, false> : rollout_vec_kernel<real, false, false>);
+    cudaFuncAttributes fa;
+    NOC_CUDA(cudaFuncGetAttributes(&fa, kern));
+    if (nthreads > fa.maxThreadsPerBlock)
+        kern = wsm ? rollout_vec_kernel_1024<real, true> : rollout_vec_kernel_1024<real, false>;
     NOC_CUDA(cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
     int grid = (int)std::min<long long>(n, 16LL * sm_count());
     kern<<<grid, nthreads, smem, st>>>(A);
